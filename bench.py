@@ -20,6 +20,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is cached in it
 
 import numpy as np  # noqa: E402
 
@@ -50,7 +51,41 @@ def parse():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--frames", type=int, default=FRAMES_PER_GPU, help="frames per GPU per step")
     ap.add_argument("--cpu-frames", type=int, default=0, help="frames in the cpu_baseline sample (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's frames) as DIR/<name>.npy, float32 / float64, < 64 MB")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 60 << 20         # array bytes of a dump: with the .npy headers below 64 MB in either unit
+DUMP_DIFFMAP_ROWS = 2048     # (frame, hypothesis) rows of the H x N diffmaps kept: 13 MB of the 1.7 GB a step writes
+DUMP_SEED = 20170721
+
+
+def dump_outputs(d, res):
+    """The arrays dsac_fetch returns for the step, as d/<name>.npy: real arrays in their own precision, integer arrays as
+    float64 (exact).  Of the diffmaps a fixed, seeded sample of rows is kept (diffmaps_rows, with their (frame, hypothesis)
+    in diffmaps_rows_index); if the per-frame arrays still exceed the budget, a fixed, seeded sample of frames is kept
+    (frame_index)."""
+    os.makedirs(d, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    nf, H = res.scores.shape
+    rows = np.sort(rng.choice(nf * H, size=min(nf * H, DUMP_DIFFMAP_ROWS), replace=False))
+    out = {"diffmaps_rows": res.diffmaps.reshape(nf * H, -1)[rows],
+           "diffmaps_rows_index": np.stack([rows // H, rows % H], 1).astype(np.float64)}
+    per_frame = {k: (a if a.dtype.kind == "f" else a.astype(np.float64)) for k, a in vars(res).items()
+                 if isinstance(a, np.ndarray) and k != "diffmaps"}
+    room = DUMP_BYTES - sum(a.nbytes for a in out.values())
+    keep = min(nf, room // sum(a.nbytes // nf for a in per_frame.values()))
+    if keep < nf:
+        frames = np.sort(rng.choice(nf, size=keep, replace=False))
+        per_frame = {k: a[frames] for k, a in per_frame.items()}
+        out["frame_index"] = frames.astype(np.float64)
+    out.update(per_frame)
+    for k, a in out.items():
+        np.save(os.path.join(d, k + ".npy"), np.ascontiguousarray(a))
 
 
 def peaks():
@@ -228,6 +263,7 @@ def main():
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the engine has no CPU path (use --impl reference for the CPU arm)")
+    E.load(build_if_missing=False)      # the library as built; the benchmark never compiles into the tree
     torch.cuda.set_device(local_rank)
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
@@ -297,7 +333,11 @@ def main():
     value = n_total * H * args.steps / (ms_total * 1e-3)
 
     # quality of the result (pose error vs the generating pose)
-    res = eng.fetch(nf)
+    dump = bool(args.dump_outputs) and rank == 0
+    res = eng.fetch(nf, want_diffmaps=dump)
+    if dump:
+        dump_outputs(args.dump_outputs, res)
+        res.diffmaps = None
     quality = {"accuracy_5cm5deg": float(res.correct.mean()), "median_rot_deg": float(np.median(res.rot_err)),
                "median_t_mm": float(np.median(res.t_err)), "candidates_per_frame": float(res.n_candidates.mean()),
                "frames_with_status": int((res.status != 0).sum())}
@@ -615,7 +655,6 @@ def main():
     barrier()
     if rank == 0:
         try:
-            subprocess.check_call(["make", "-C", os.path.join(ROOT, "apps"), "-s"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
             with tempfile.TemporaryDirectory() as d:
                 cmd = [os.path.join(ROOT, "apps", "test_ransac_softam"), "-frames", "1000", "-batch", "250", "-gpus", str(world)]
                 subprocess.run(cmd, cwd=d, capture_output=True, text=True, timeout=300)   # first run: engine creation, page-in

@@ -6,6 +6,7 @@ cpu_baseline / --impl reference leg.  Never imported by the product package dsac
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -419,19 +420,26 @@ _variants = {}
 def variant_lib(variant):
     """A differently COMPILED build of the same oracle sources, for the CPU timing arm only (bench.py): "parity" = the -O2
     -ffp-contract=off library the tests use; "perf" = -O3 -march=x86-64-v3 -fopenmp; "native" / "ofast" = -O3 / -Ofast
-    -march=native, built on the calling box (BASELINE.md section 3).  Returns (CDLL, flags description) or (None, why)."""
+    -march=native, built on the calling machine into a temporary directory (BASELINE.md section 3).  Returns (CDLL, flags
+    description) or (None, why)."""
     if variant == "parity":
         return lib(), "-O2 -ffp-contract=off (parity build)"
     if variant in _variants:
         return _variants[variant]
     target = {"perf": "libdsac_oracle_perf.so", "native": "libdsac_oracle_native.so", "ofast": "libdsac_oracle_ofast.so"}[variant]
     flags = {"perf": "-O3 -march=x86-64-v3 -fopenmp", "native": "-O3 -march=native -fopenmp", "ofast": "-Ofast -march=native -fopenmp"}[variant]
-    path = os.path.join(_HERE, target)
     try:
-        if variant != "perf" or not os.path.exists(path):
-            subprocess.check_call(["make", "-C", _HERE, "-s", "-B" if variant != "perf" else "-s", target], stdout=subprocess.DEVNULL,
-                                  stderr=subprocess.DEVNULL)
-        l = C.CDLL(path)
+        if variant == "perf":
+            path = os.path.join(_HERE, target)
+            if not os.path.exists(path):
+                subprocess.check_call(["make", "-C", _HERE, "-s", target], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            l = C.CDLL(path)
+        else:
+            with tempfile.TemporaryDirectory() as d:   # the library stays mapped once the directory is gone
+                path = os.path.join(d, target)
+                subprocess.check_call(["make", "-C", _HERE, "-s", "VARIANT_DIR=" + d, path], stdout=subprocess.DEVNULL,
+                                      stderr=subprocess.DEVNULL)
+                l = C.CDLL(path)
         l.orc_bench_forward.restype = C.c_double
         _variants[variant] = (l, flags)
     except Exception as e:   # no compiler on this box, or an instruction set this CPU lacks

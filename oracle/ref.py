@@ -1,6 +1,7 @@
 """ctypes binding of oracle/_ref: the reference's OWN pipeline sources compiled unmodified (oracle/Makefile, oracle/shim,
-oracle/ref_harness).  TEST INFRASTRUCTURE ONLY, and only where /root/reference exists (this container, not the GPU box):
-tests/test_oracle_vs_ref.py pins the oracle to it and tests/golden/make_ref_golden.py freezes its outputs as fixtures.
+oracle/ref_harness).  TEST INFRASTRUCTURE ONLY, and only where the reference's sources are present:
+tests/golden/make_ref_golden.py and make_ref_cases_golden.py freeze its outputs as the fixtures that
+tests/test_oracle_vs_ref.py compares the oracle against (write_dataset() alone needs no reference).
 """
 import ctypes as C
 import os
