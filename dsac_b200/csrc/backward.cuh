@@ -13,6 +13,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include "device_block.h"
 #include "pose_math.cuh"
 #include "refine.cuh"
 
@@ -25,10 +26,9 @@ constexpr int BW_MAX_OBJ_PIX = 16;                       // ceil(1600 / skip) wi
 constexpr int BW_JOBS = 12 + BW_MAX_OBJ_PIX * 6;         // refine jobs per frame (dRefineHyp + dRefineObj)
 
 struct BackwardScratch {
-    void* buf = nullptr;
-    size_t bytes = 0;
+    DeviceBlock block;               // grow-only, owned by the engine
     int n_cap = 0;
-    // carved from buf
+    // carved from block
     int32_t* job_frame = nullptr;    // [n][BW_JOBS]
     double* job_init = nullptr;      // [n][BW_JOBS][6]
     int32_t* job_pert = nullptr;     // [n][BW_JOBS][2]
@@ -46,10 +46,6 @@ struct BackwardScratch {
     double* part = nullptr;          // [n][groups][N*3] partial rows of k_dscore
     int groups = 1;
 };
-inline void backward_scratch_free(BackwardScratch* s) {
-    if (s->buf) cudaFree(s->buf);
-    *s = BackwardScratch();
-}
 
 // Hypothesis(cv2our(pose)).getRodVecAndTrans()  (Hypothesis.cpp:274-290)
 __device__ __forceinline__ void jp6_from_cv_dev(const double pose[6], double out[6]) {

@@ -18,6 +18,7 @@
 
 #include "../../include/dsac_b200.h"
 #include "backward.cuh"
+#include "device_block.h"
 #include "kernels.cuh"
 #include "refine.cuh"
 #include "sampler_split.cuh"
@@ -26,6 +27,21 @@
 using namespace dsac;
 
 static std::string g_create_error;
+
+// One lane of the split sampler (sampler_split.cuh): the streams, events, queue counters and acceptance statistics of one
+// pass.  Lane 0 runs its generator on the caller's stream; lane 1, the second half of a large batch (forward_split), on `main`.
+struct K1Lane {
+    cudaStream_t main = nullptr;                  // lane 1 only
+    cudaStream_t side = nullptr;                  // k1_filter (and k1_solve), next to the generator on the lane's stream
+    cudaStream_t side2 = nullptr;                 // k1_solve, when it runs next to the following set's filter
+    cudaEvent_t ev_filt[K1S_MAX_SETS] = {};       // filter of launch set i done
+    cudaEvent_t ev_solve[K1S_MAX_SETS] = {};      // solve of launch set i done
+    cudaEvent_t ev_gen[K1S_MAX_SETS] = {};        // generation of launch set i done
+    cudaEvent_t ev_round = nullptr;               // last solve of a round done
+    int* counters = nullptr;                      // wq_n[K1S_MAX_SETS], fq_n[K1S_MAX_SETS]
+    unsigned long long* stats = nullptr;          // [2][2]: candidates / hypotheses of finished streams, by call parity
+    unsigned long long calls = 0;
+};
 
 struct dsac_engine {
     dsac_config cfg;
@@ -36,12 +52,17 @@ struct dsac_engine {
     void* hook_user = nullptr;
     dsac_score_backward_hook bw_hook = nullptr;
     void* bw_hook_user = nullptr;
-    double* d_ext_g = nullptr;      // [n][H][N] dScore/dDiffMap from the backward hook (grow-only)
-    size_t ext_g_count = 0;
     cudaEvent_t ev_fwd = nullptr;   // recorded after the last forward launch: the backward waits on it
-    double* d_kabsch = nullptr;     // dsac_kabsch: inputs and outputs in one grow-only block
-    size_t kabsch_bytes = 0;
     int sm_count = 148;
+    // device memory for the engine's lifetime (dev_alloc): freed by dsac_engine_destroy
+    std::vector<void*> owned;
+    // grow-only device memory, (re)allocated on use
+    DeviceBlock ext_g;              // [n][H][N] dScore/dDiffMap from the backward hook, then [n][H] clamped output gradients
+    DeviceBlock kabsch;             // dsac_kabsch: inputs and outputs in one block
+    BackwardScratch bw;             // dsac_backward (bw.block)
+    DeviceBlock ra;                 // refine-all (DSAC variant): d_ra_* below are carved from it for ra_jobs jobs
+    DeviceBlock ra_imap;            // refine-all inlier maps
+    std::vector<DeviceBlock> bw_pool;   // device buffers of dsac_backward_dsac, kept across calls
     // inputs (device copies for the host-buffer entry point)
     int16_t* d_coords = nullptr;
     int32_t* d_pix = nullptr;
@@ -52,7 +73,6 @@ struct dsac_engine {
     int cur_pix_shared = 0;
     const double* cur_gt = nullptr;
     int cur_n = 0;
-    int k1_slots = 296;             // resident k_sample CTAs on this GPU (SMs x CTAs/SM), set at creation
     int dsac_n = 0;                 // frames of the last dsac_forward_dsac (0: none), for dsac_backward_dsac
     long long cur_frame0 = 0;
     // state
@@ -63,10 +83,9 @@ struct dsac_engine {
     int32_t* d_cand_idx = nullptr;
     long long* d_stream_ncand = nullptr;
     unsigned long long* d_stream_endpos = nullptr;
-    // refine-all (DSAC variant) buffers, allocated on first use
     int32_t* d_ra_frame = nullptr; double* d_ra_pose = nullptr; double* d_ra_loss = nullptr; double* d_ra_rot = nullptr;
-    double* d_ra_t = nullptr; int32_t* d_ra_correct = nullptr; int32_t* d_ra_steps = nullptr; int32_t* d_ra_imap = nullptr;
-    size_t ra_jobs = 0, ra_imap_jobs = 0;
+    double* d_ra_t = nullptr; int32_t* d_ra_correct = nullptr; int32_t* d_ra_steps = nullptr;
+    size_t ra_jobs = 0;
     uint32_t* d_status = nullptr;
     unsigned long long* d_fragile = nullptr;
     unsigned long long* d_phase = nullptr;   // K1 per-phase cycle counters (DSAC_K1_TIMERS=1), else null
@@ -86,22 +105,17 @@ struct dsac_engine {
     unsigned int* d_frame_counter = nullptr;
     long long* h_stream_ncand = nullptr;   // [max_frames][n_streams], pinned (so that a submitted pass stays asynchronous)
     dsac_forward_out* pending_out = nullptr;   // results of a submitted, not yet awaited pass
-    int pending_n = 0, pending_chunks = 0;
-    BackwardScratch bw;
-    std::vector<std::pair<void*, size_t>> bw_pool;   // device buffers of dsac_backward_dsac, kept across calls
-    cudaStream_t pipe[4] = {nullptr, nullptr, nullptr, nullptr};   // chunked H2D / compute / D2H pipeline of dsac_forward
-    // tail split (dsac_set_tail_split): the whole sampler waves of a batch run on a high-priority side stream, the
-    // frames of the last, partial wave on the caller's stream, so that scoring / refinement of the first part fill
-    // the SMs the partial wave leaves idle
-    cudaStream_t hi = nullptr;
+    int pending_n = 0;
+    bool pending = false;
+    cudaStream_t stream = nullptr;          // the engine's stream: host-buffer passes and the backward passes
+    cudaStream_t kabsch_stream = nullptr;   // dsac_kabsch
+    // two lanes (forward_split): fork / join of lane 1 with the caller's stream
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    int tail_split = 1;
+    int tail_split = 1;             // dsac_set_tail_split
     // split sampler (sampler_split.cuh): per-stream state and round buffers, sized at creation
-    int k1_mode = 1;                // 1: round-based pipeline of flat kernels; 0: monolithic k_sample (DSAC_K1_MODE=mono)
-    int k1_rounds = 3, k1_cap = 0;   // rounds 0..2 finish every stream of the benchmark batches; a straggler continues in k_sample (resume). 5 rounds = 6 empty launches per pass (measured +0.02 ms)
-    bool k1_rounds_fixed = false;   // DSAC_K1_ROUNDS given
+    int k1_cap = 0;
     int k1_filter_grid = 0, k1_solve_grid = 0;
-    unsigned long long k1_calls = 0;
+    K1Lane lane[2];
     K1SlotState* d_k1_state = nullptr;
     CellRec* d_k1_celltab = nullptr;
     uint2* d_k1_cells = nullptr;
@@ -110,33 +124,12 @@ struct dsac_engine {
     double* d_k1_pose = nullptr;
     uint2* d_k1_wq = nullptr;
     uint32_t* d_k1_fq = nullptr;
-    int* d_k1_counters = nullptr;                 // wq_n[K1S_MAX_ROUNDS], fq_n[K1S_MAX_ROUNDS]
-    unsigned long long* d_k1_stats = nullptr;     // [2][2]: candidates / hypotheses of finished streams, by call parity
     unsigned long long* d_k1_dbg = nullptr;       // [K1S_MAX_ROUNDS][4] (DSAC_K1_DEBUG=1 or dsac_sampler_profile), else null
     // dsac_sampler_profile: CUDA events between the sampler's launches of the last forward pass
     int k1_profile = 0;
     std::vector<cudaEvent_t> k1_ev;               // event i is recorded after launch i (event 0 before the first)
     std::vector<int> k1_ev_kind;                  // 0 cells/slot (integer generation + selection), 1 filter, 2 solve, 3 resume tail
     int k1_ev_n = 0;
-    // generator / filter overlap: k1_slot runs on the caller's stream, k1_filter + k1_solve on this side stream
-    cudaStream_t k1_side = nullptr;
-    cudaStream_t k1_side2 = nullptr;              // k1_solve, when it runs next to the following set's filter (overlap mode 2)
-    cudaEvent_t k1_ev_filt[K1S_MAX_SETS] = {};    // filter of launch set i done
-    cudaEvent_t k1_ev_solve[K1S_MAX_SETS] = {};   // solve of launch set i done
-    cudaEvent_t k1_ev_gen[K1S_MAX_SETS] = {};     // generation of launch set i done
-    cudaEvent_t k1_ev_round = nullptr;            // last solve of a round done
-    // a second, independent set of the per-pass sampler resources: a large batch runs as two concurrent half-batches (forward_split)
-    struct K1Lane {
-        cudaStream_t main = nullptr, side = nullptr, side2 = nullptr;
-        cudaEvent_t ev_filt[K1S_MAX_SETS] = {}, ev_solve[K1S_MAX_SETS] = {}, ev_gen[K1S_MAX_SETS] = {}, ev_round = nullptr;
-        int* counters = nullptr;
-        unsigned long long* stats = nullptr;
-        unsigned long long calls = 0;
-    } lane1;
-    int k1_lanes = 1;                             // DSAC_K1_LANES: 0 = never split a batch into two lanes
-    int k1_overlap = 1;
-    bool k1_overlap_fixed = false;                // DSAC_K1_OVERLAP given
-    int k1_solve_batch = 0;                       // 1: one k1_solve per round over the flagged candidates of all its launch sets (measured SLOWER, 3.07 vs 2.92 ms per step: a per-set solve runs beside the next set's generator, a per-round one runs alone)
     K1SlotState* d_k1_vstate = nullptr;           // k1_spec: virtual slots of the speculative first round (few streams)
     uint2* d_k1_vcells = nullptr;
     uint32_t* d_k1_vendw = nullptr;
@@ -147,11 +140,25 @@ struct dsac_engine {
     int k1_pipe = 0;                              // DSAC_K1_PIPE=1: chained generator for 9 .. ~190 streams (experimental, off by default)
     int k1_slot_capacity = 0;                     // CTAs of k1_pipe / k1_slot (256 threads) the GPU holds at once
     int k1_spec_slots = 0;                        // streams the scratch above was sized for (0: speculative round off)
-    int k1_solve_group4 = 1;                      // DSAC_K1_SOLVE4: four lanes per flagged candidate for a few streams
     int k1_slot_threads = 0;                      // DSAC_K1_SLOT_THREADS: 256 / 512 / 1024 (0: by the number of streams)
-    int k1_fused = 0;                             // 1: filter of set k and generator of set k+1 in one warp-specialised kernel (k1_fused)
     int k1_wq_stride = 0;
 };
+
+// Rounds of the split sampler per pass: rounds 0..2 finish every stream of the benchmark batches; a straggler continues in
+// k_sample (resume).  5 rounds = 6 empty launches per pass (measured +0.02 ms).
+constexpr int K1_ROUNDS = 3;
+
+// Engine-lifetime device memory: recorded in e->owned and freed by dsac_engine_destroy.
+template <typename T>
+static cudaError_t dev_alloc(dsac_engine* e, T** p, size_t bytes) {
+    const cudaError_t st = cudaMalloc(p, bytes);
+    if (st != cudaSuccess) {
+        *p = nullptr;
+        return st;
+    }
+    e->owned.push_back(*p);
+    return cudaSuccess;
+}
 
 static int fail(dsac_engine* e, int code, const char* fmt, ...) {
     char buf[512];
@@ -210,21 +217,16 @@ int dsac_engine_config(const dsac_engine* e, dsac_config* out) {
 void dsac_engine_destroy(dsac_engine* e) {
     if (!e) return;
     cudaSetDevice(e->cfg.device);
-    for (cudaStream_t st : e->pipe)
-        if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
-    if (e->hi) { cudaStreamSynchronize(e->hi); cudaStreamDestroy(e->hi); }
-    if (e->ev_fork) cudaEventDestroy(e->ev_fork);
-    if (e->ev_join) cudaEventDestroy(e->ev_join);
-    if (e->ev_fwd) cudaEventDestroy(e->ev_fwd);
-    if (e->d_ext_g) cudaFree(e->d_ext_g);
-    if (e->d_kabsch) cudaFree(e->d_kabsch);
+    const cudaStream_t streams[] = {e->stream, e->kabsch_stream, e->lane[0].side, e->lane[0].side2,
+                                    e->lane[1].main, e->lane[1].side, e->lane[1].side2};
+    for (cudaStream_t st : streams)
+        if (st) cudaStreamSynchronize(st);
     if (e->d_phase) {
         unsigned long long h[16];
         if (cudaMemcpy(h, e->d_phase, sizeof(h), cudaMemcpyDeviceToHost) == cudaSuccess)
             fprintf(stderr, "[dsac K1 thread-0 cycles] A1 gen %llu  A2 bounds %llu  B filter %llu  C queue %llu  D full %llu  E advance %llu\n"
                             "[dsac k1_slot thread-0 cycles] regenerate+decode %llu  scan %llu  walk %llu  starts %llu  write %llu  leftover %llu\n",
                     h[0], h[1], h[2], h[3], h[4], h[5], h[8], h[9], h[10], h[11], h[12], h[13]);
-        cudaFree(e->d_phase);
     }
     if (e->d_k1_dbg && e->d_k1_spec_result && e->k1_spec_slots > 0) {
         int h[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -239,40 +241,21 @@ void dsac_engine_destroy(dsac_engine* e) {
                 fprintf(stderr, "[dsac K1 split, last call] round %d: %llu active streams, %llu candidates, %llu flagged, %llu accepted\n", r,
                         h[r * 4], h[r * 4 + 1], h[r * 4 + 2], h[r * 4 + 3]);
     }
-    for (cudaEvent_t ev : e->k1_ev) cudaEventDestroy(ev);
-    if (e->k1_side) { cudaStreamSynchronize(e->k1_side); cudaStreamDestroy(e->k1_side); }
-    if (e->k1_side2) { cudaStreamSynchronize(e->k1_side2); cudaStreamDestroy(e->k1_side2); }
-    for (cudaEvent_t ev : e->k1_ev_filt) if (ev) cudaEventDestroy(ev);
-    for (cudaEvent_t ev : e->k1_ev_solve) if (ev) cudaEventDestroy(ev);
-    for (cudaEvent_t ev : e->k1_ev_gen) if (ev) cudaEventDestroy(ev);
-    if (e->k1_ev_round) cudaEventDestroy(e->k1_ev_round);
-    {
-        dsac_engine::K1Lane& L = e->lane1;
-        for (cudaStream_t st : {L.main, L.side, L.side2}) if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
-        for (int i = 0; i < K1S_MAX_SETS; i++) {
-            if (L.ev_filt[i]) cudaEventDestroy(L.ev_filt[i]);
-            if (L.ev_solve[i]) cudaEventDestroy(L.ev_solve[i]);
-            if (L.ev_gen[i]) cudaEventDestroy(L.ev_gen[i]);
-        }
+    for (cudaStream_t st : streams)
+        if (st) cudaStreamDestroy(st);
+    for (K1Lane& L : e->lane) {
+        for (int i = 0; i < K1S_MAX_SETS; i++)
+            for (cudaEvent_t ev : {L.ev_filt[i], L.ev_solve[i], L.ev_gen[i]})
+                if (ev) cudaEventDestroy(ev);
         if (L.ev_round) cudaEventDestroy(L.ev_round);
-        if (L.counters) cudaFree(L.counters);
-        if (L.stats) cudaFree(L.stats);
     }
-    void* k1ptrs[] = {e->d_k1_chain, e->d_k1_spec_table, e->d_k1_vstate, e->d_k1_vcells, e->d_k1_vendw, e->d_k1_spec_result, e->d_k1_state, e->d_k1_celltab, e->d_k1_cells, e->d_k1_endw, e->d_k1_accbits, e->d_k1_pose, e->d_k1_wq,
-                      e->d_k1_fq, e->d_k1_counters, e->d_k1_stats, e->d_k1_dbg};
-    for (void* p : k1ptrs)
-        if (p) cudaFree(p);
-    void* ptrs[] = {e->d_coords, e->d_pix, e->d_gt, e->d_perm, e->d_hyp_pose, e->d_hyp_P, e->d_img_idx, e->d_cand_idx,
-                    e->d_stream_ncand, e->d_stream_endpos, e->d_ra_frame, e->d_ra_pose, e->d_ra_loss, e->d_ra_rot, e->d_ra_t,
-                    e->d_ra_correct, e->d_ra_steps, e->d_ra_imap, e->d_status, e->d_fragile, e->d_diffmaps, e->d_scores, e->d_sf, e->d_entropy,
-                    e->d_avg, e->d_ref, e->d_inlier_map, e->d_steps_done, e->d_n_perm, e->d_loss, e->d_rot_err,
-                    e->d_t_err, e->d_correct, e->d_frame_counter};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
+    for (cudaEvent_t ev : {e->ev_fork, e->ev_join, e->ev_fwd})
+        if (ev) cudaEventDestroy(ev);
+    for (cudaEvent_t ev : e->k1_ev) cudaEventDestroy(ev);
+    for (void* p : e->owned) cudaFree(p);
+    for (DeviceBlock* b : {&e->ext_g, &e->kabsch, &e->bw.block, &e->ra, &e->ra_imap}) b->release();
+    for (DeviceBlock& b : e->bw_pool) b.release();
     if (e->h_stream_ncand) cudaFreeHost(e->h_stream_ncand);
-    backward_scratch_free(&e->bw);
-    for (auto& slot : e->bw_pool)
-        if (slot.first) cudaFree(slot.first);
     delete e;
 }
 
@@ -312,36 +295,36 @@ int dsac_engine_create(const dsac_config* cfg, dsac_engine** out) {
     CUC(cudaGetDeviceProperties(&prop, cfg->device));
     e->sm_count = prop.multiProcessorCount;
     const size_t n = (size_t)cfg->max_frames, H = (size_t)cfg->n_hyps, N = DSAC_N;
-    CUC(cudaMalloc(&e->d_coords, n * N * 3 * sizeof(int16_t)));
-    CUC(cudaMalloc(&e->d_pix, n * N * 2 * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_gt, n * 12 * sizeof(double)));
-    CUC(cudaMalloc(&e->d_perm, (size_t)std::max(1, cfg->ref_steps) * N * sizeof(uint16_t)));
-    CUC(cudaMalloc(&e->d_hyp_pose, n * H * 6 * sizeof(double)));
-    CUC(cudaMalloc(&e->d_hyp_P, n * H * 12 * sizeof(float)));
-    CUC(cudaMalloc(&e->d_img_idx, n * H * 4 * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_cand_idx, n * H * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_stream_ncand, n * cfg->n_streams * sizeof(long long)));
-    CUC(cudaMalloc(&e->d_stream_endpos, n * cfg->n_streams * sizeof(unsigned long long)));
-    CUC(cudaMalloc(&e->d_status, n * sizeof(uint32_t)));
-    CUC(cudaMalloc(&e->d_fragile, sizeof(unsigned long long)));
-    if (cfg->write_diffmaps) CUC(cudaMalloc(&e->d_diffmaps, n * H * N * sizeof(float)));
-    CUC(cudaMalloc(&e->d_scores, n * H * sizeof(double)));
-    CUC(cudaMalloc(&e->d_sf, n * H * sizeof(double)));
-    CUC(cudaMalloc(&e->d_entropy, n * sizeof(double)));
-    CUC(cudaMalloc(&e->d_avg, n * 6 * sizeof(double)));
-    CUC(cudaMalloc(&e->d_ref, n * 6 * sizeof(double)));
-    CUC(cudaMalloc(&e->d_inlier_map, n * N * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_steps_done, n * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_n_perm, n * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_loss, n * sizeof(double)));
-    CUC(cudaMalloc(&e->d_rot_err, n * sizeof(double)));
-    CUC(cudaMalloc(&e->d_t_err, n * sizeof(double)));
-    CUC(cudaMalloc(&e->d_correct, n * sizeof(int32_t)));
-    CUC(cudaMalloc(&e->d_frame_counter, n * sizeof(unsigned int)));
+    CUC(dev_alloc(e, &e->d_coords, n * N * 3 * sizeof(int16_t)));
+    CUC(dev_alloc(e, &e->d_pix, n * N * 2 * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_gt, n * 12 * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_perm, (size_t)std::max(1, cfg->ref_steps) * N * sizeof(uint16_t)));
+    CUC(dev_alloc(e, &e->d_hyp_pose, n * H * 6 * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_hyp_P, n * H * 12 * sizeof(float)));
+    CUC(dev_alloc(e, &e->d_img_idx, n * H * 4 * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_cand_idx, n * H * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_stream_ncand, n * cfg->n_streams * sizeof(long long)));
+    CUC(dev_alloc(e, &e->d_stream_endpos, n * cfg->n_streams * sizeof(unsigned long long)));
+    CUC(dev_alloc(e, &e->d_status, n * sizeof(uint32_t)));
+    CUC(dev_alloc(e, &e->d_fragile, sizeof(unsigned long long)));
+    if (cfg->write_diffmaps) CUC(dev_alloc(e, &e->d_diffmaps, n * H * N * sizeof(float)));
+    CUC(dev_alloc(e, &e->d_scores, n * H * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_sf, n * H * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_entropy, n * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_avg, n * 6 * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_ref, n * 6 * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_inlier_map, n * N * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_steps_done, n * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_n_perm, n * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_loss, n * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_rot_err, n * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_t_err, n * sizeof(double)));
+    CUC(dev_alloc(e, &e->d_correct, n * sizeof(int32_t)));
+    CUC(dev_alloc(e, &e->d_frame_counter, n * sizeof(unsigned int)));
     CUC(cudaMemset(e->d_frame_counter, 0, n * sizeof(unsigned int)));
     CUC(cudaMemset(e->d_fragile, 0, sizeof(unsigned long long)));
     if (getenv("DSAC_K1_TIMERS")) {
-        CUC(cudaMalloc(&e->d_phase, 16 * sizeof(unsigned long long)));
+        CUC(dev_alloc(e, &e->d_phase, 16 * sizeof(unsigned long long)));
         CUC(cudaMemset(e->d_phase, 0, 16 * sizeof(unsigned long long)));
     }
     CUC(cudaMemset(e->d_status, 0, n * sizeof(uint32_t)));
@@ -372,17 +355,8 @@ int dsac_engine_create(const dsac_config* cfg, dsac_engine** out) {
     // need not pick the split the launch bounds were written for).  k_sample is left to the default: it spills to
     // local memory and measured 5 % slower with the largest carve-out (3.39 vs 3.24 ms), i.e. with the smallest L1.
     CUC(cudaFuncSetAttribute(k_refine, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    if (const char* co = getenv("DSAC_K1_CARVEOUT")) CUC(cudaFuncSetAttribute(k_sample, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(co)));
-    {
-        int per_sm = 0, sms = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sample, K1_THREADS, sizeof(K1Smem));
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, cfg->device);
-        if (per_sm > 0 && sms > 0) e->k1_slots = per_sm * sms;
-    }
     CUC(cudaMallocHost(&e->h_stream_ncand, n * cfg->n_streams * sizeof(long long)));
-    if (const char* m = getenv("DSAC_K1_MODE")) e->k1_mode = (strcmp(m, "mono") == 0) ? 0 : 1;
-    if (const char* r = getenv("DSAC_K1_ROUNDS")) { e->k1_rounds = std::max(1, std::min(K1S_MAX_ROUNDS - 1, atoi(r))); e->k1_rounds_fixed = true; }
-    if (e->k1_mode) {
+    {
         const size_t T = (size_t)cfg->n_streams, slots = n * T;
         const int quota_max = (cfg->n_hyps + cfg->n_streams - 1) / cfg->n_streams;
         // few streams (single-frame latency): the first round takes 115 % of the expected need, so the capacity is larger
@@ -391,16 +365,15 @@ int dsac_engine_create(const dsac_config* cfg, dsac_engine** out) {
         cap = (cap + 1023) & ~1023;     // a round is generated in portions of cap / 4, themselves multiples of 256
         e->k1_cap = cap;
         e->k1_wq_stride = (int)(slots * 128);
-        CUC(cudaMalloc(&e->d_k1_state, slots * sizeof(K1SlotState)));
-        CUC(cudaMalloc(&e->d_k1_celltab, n * N * sizeof(CellRec)));
-        CUC(cudaMalloc(&e->d_k1_cells, slots * cap * sizeof(uint2)));
-        CUC(cudaMalloc(&e->d_k1_endw, slots * cap * sizeof(uint32_t)));
-        CUC(cudaMalloc(&e->d_k1_accbits, slots * (cap / 32) * sizeof(uint32_t)));
-        CUC(cudaMalloc(&e->d_k1_pose, slots * cap * 6 * sizeof(double)));
-        CUC(cudaMalloc(&e->d_k1_wq, (size_t)K1S_MAX_SETS * slots * 128 * sizeof(uint2)));
-        CUC(cudaMalloc(&e->d_k1_fq, 2 * slots * cap * sizeof(uint32_t)));   // two regions: the filter of set k+1 writes one while the solve of set k reads the other
-        CUC(cudaMalloc(&e->d_k1_counters, 2 * K1S_MAX_SETS * sizeof(int)));
-        CUC(cudaMalloc(&e->d_k1_chain, slots * (K1Q_MAX_WIN + 1) * 4 * sizeof(uint32_t)));
+        CUC(dev_alloc(e, &e->d_k1_state, slots * sizeof(K1SlotState)));
+        CUC(dev_alloc(e, &e->d_k1_celltab, n * N * sizeof(CellRec)));
+        CUC(dev_alloc(e, &e->d_k1_cells, slots * cap * sizeof(uint2)));
+        CUC(dev_alloc(e, &e->d_k1_endw, slots * cap * sizeof(uint32_t)));
+        CUC(dev_alloc(e, &e->d_k1_accbits, slots * (cap / 32) * sizeof(uint32_t)));
+        CUC(dev_alloc(e, &e->d_k1_pose, slots * cap * 6 * sizeof(double)));
+        CUC(dev_alloc(e, &e->d_k1_wq, (size_t)K1S_MAX_SETS * slots * 128 * sizeof(uint2)));
+        CUC(dev_alloc(e, &e->d_k1_fq, 2 * slots * cap * sizeof(uint32_t)));   // two regions: the filter of set k+1 writes one while the solve of set k reads the other
+        CUC(dev_alloc(e, &e->d_k1_chain, slots * (K1Q_MAX_WIN + 1) * 4 * sizeof(uint32_t)));
         CUC(cudaMemset(e->d_k1_chain, 0, slots * (K1Q_MAX_WIN + 1) * 4 * sizeof(uint32_t)));
         {
             int per_sm = 0;
@@ -413,35 +386,22 @@ int dsac_engine_create(const dsac_config* cfg, dsac_engine** out) {
             if (const char* sv = getenv("DSAC_K1_SPEC")) want = atoi(sv);
             if (want) {
                 const size_t ss = std::min<size_t>(slots, 8);    // measured: 8 frames x 1 stream 0.546 -> 0.481 ms per step, 16 frames 0.565 -> 0.571 (1360 window CTAs: no longer one wave)
-                CUC(cudaMalloc(&e->d_k1_vstate, ss * K1P_VPER * sizeof(K1SlotState)));
-                CUC(cudaMalloc(&e->d_k1_vcells, ss * K1P_VPER * K1P_CAPW * sizeof(uint2)));
-                CUC(cudaMalloc(&e->d_k1_vendw, ss * K1P_VPER * K1P_CAPW * sizeof(uint32_t)));
-                CUC(cudaMalloc(&e->d_k1_spec_result, ss * sizeof(int)));
+                CUC(dev_alloc(e, &e->d_k1_vstate, ss * K1P_VPER * sizeof(K1SlotState)));
+                CUC(dev_alloc(e, &e->d_k1_vcells, ss * K1P_VPER * K1P_CAPW * sizeof(uint2)));
+                CUC(dev_alloc(e, &e->d_k1_vendw, ss * K1P_VPER * K1P_CAPW * sizeof(uint32_t)));
+                CUC(dev_alloc(e, &e->d_k1_spec_result, ss * sizeof(int)));
                 CUC(cudaMemset(e->d_k1_spec_result, 0, ss * sizeof(int)));
-                CUC(cudaMalloc(&e->d_k1_spec_table, ss * K1P_TABLE * sizeof(int)));
+                CUC(dev_alloc(e, &e->d_k1_spec_table, ss * K1P_TABLE * sizeof(int)));
                 e->k1_spec_slots = (int)ss;
             }
         }
-        {   // the fp64 kernels get the higher priority: when a generator launch and a filter launch become ready together,
-            // the persistent filter CTAs are placed first and the generator's CTAs fill the registers they leave free
-            int least = 0, greatest = 0;
-            CUC(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-            int prio = greatest;
-            if (const char* pr = getenv("DSAC_K1_SIDE_PRIO")) prio = atoi(pr) ? greatest : least;
-            CUC(cudaStreamCreateWithPriority(&e->k1_side, cudaStreamNonBlocking, prio));
-            CUC(cudaStreamCreateWithPriority(&e->k1_side2, cudaStreamNonBlocking, prio));
-            for (int i = 0; i < K1S_MAX_SETS; i++) {
-                CUC(cudaEventCreateWithFlags(&e->k1_ev_filt[i], cudaEventDisableTiming));
-                CUC(cudaEventCreateWithFlags(&e->k1_ev_solve[i], cudaEventDisableTiming));
-            }
-        }
-        for (int i = 0; i < K1S_MAX_SETS; i++) CUC(cudaEventCreateWithFlags(&e->k1_ev_gen[i], cudaEventDisableTiming));
-        CUC(cudaEventCreateWithFlags(&e->k1_ev_round, cudaEventDisableTiming));
-        {   // the second lane (forward_split: two concurrent half-batches)
-            int least = 0, greatest = 0;
-            CUC(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-            dsac_engine::K1Lane& L = e->lane1;
-            CUC(cudaStreamCreateWithFlags(&L.main, cudaStreamNonBlocking));
+        // the lanes.  The fp64 kernels get the higher priority: when a generator launch and a filter launch become ready
+        // together, the persistent filter CTAs are placed first and the generator's CTAs fill the registers they leave free
+        int least = 0, greatest = 0;
+        CUC(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        for (int l = 0; l < 2; l++) {
+            K1Lane& L = e->lane[l];
+            if (l == 1) CUC(cudaStreamCreateWithFlags(&L.main, cudaStreamNonBlocking));
             CUC(cudaStreamCreateWithPriority(&L.side, cudaStreamNonBlocking, greatest));
             CUC(cudaStreamCreateWithPriority(&L.side2, cudaStreamNonBlocking, greatest));
             for (int i = 0; i < K1S_MAX_SETS; i++) {
@@ -450,20 +410,12 @@ int dsac_engine_create(const dsac_config* cfg, dsac_engine** out) {
                 CUC(cudaEventCreateWithFlags(&L.ev_gen[i], cudaEventDisableTiming));
             }
             CUC(cudaEventCreateWithFlags(&L.ev_round, cudaEventDisableTiming));
-            CUC(cudaMalloc(&L.counters, 2 * K1S_MAX_SETS * sizeof(int)));
-            CUC(cudaMalloc(&L.stats, 4 * sizeof(unsigned long long)));
+            CUC(dev_alloc(e, &L.counters, 2 * K1S_MAX_SETS * sizeof(int)));
+            CUC(dev_alloc(e, &L.stats, 4 * sizeof(unsigned long long)));
             CUC(cudaMemset(L.stats, 0, 4 * sizeof(unsigned long long)));
-            if (const char* ln = getenv("DSAC_K1_LANES")) e->k1_lanes = atoi(ln);
         }
-        if (const char* ov = getenv("DSAC_K1_OVERLAP")) { e->k1_overlap = atoi(ov); e->k1_overlap_fixed = true; }
-        if (const char* fu = getenv("DSAC_K1_FUSED")) e->k1_fused = atoi(fu);
         if (const char* stt = getenv("DSAC_K1_SLOT_THREADS")) e->k1_slot_threads = atoi(stt);
-        if (const char* s4 = getenv("DSAC_K1_SOLVE4")) e->k1_solve_group4 = atoi(s4);
-        if (const char* sb = getenv("DSAC_K1_SOLVE_BATCH")) e->k1_solve_batch = atoi(sb);
-        CUC(cudaFuncSetAttribute(k1_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(K1XSmem)));
-        CUC(cudaMalloc(&e->d_k1_stats, 4 * sizeof(unsigned long long)));
-        CUC(cudaMemset(e->d_k1_stats, 0, 4 * sizeof(unsigned long long)));
-        if (getenv("DSAC_K1_DEBUG")) CUC(cudaMalloc(&e->d_k1_dbg, K1S_MAX_ROUNDS * 4 * sizeof(unsigned long long)));
+        if (getenv("DSAC_K1_DEBUG")) CUC(dev_alloc(e, &e->d_k1_dbg, K1S_MAX_ROUNDS * 4 * sizeof(unsigned long long)));
         CUC(cudaFuncSetAttribute(k1_filter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(K1FSmem)));
         int per_sm = 0;
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k1_filter, K1F_THREADS, sizeof(K1FSmem));
@@ -471,19 +423,12 @@ int dsac_engine_create(const dsac_config* cfg, dsac_engine** out) {
         per_sm = 0;
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k1_solve, K1V_THREADS, 0);
         e->k1_solve_grid = std::max(1, per_sm) * e->sm_count;
-        if (const char* g = getenv("DSAC_K1_FILTER_GRID")) e->k1_filter_grid = std::max(1, atoi(g));
-        if (const char* g = getenv("DSAC_K1_SOLVE_GRID")) e->k1_solve_grid = std::max(1, atoi(g));
     }
-    for (int i = 0; i < 4; i++) CUC(cudaStreamCreateWithFlags(&e->pipe[i], cudaStreamNonBlocking));
-    {
-        int least = 0, greatest = 0;
-        CUC(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-        CUC(cudaStreamCreateWithPriority(&e->hi, cudaStreamNonBlocking, greatest));
-        CUC(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-        CUC(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
-        CUC(cudaEventCreateWithFlags(&e->ev_fwd, cudaEventDisableTiming));
-        if (const char* ts = getenv("DSAC_TAIL_SPLIT")) e->tail_split = atoi(ts);
-    }
+    CUC(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
+    CUC(cudaStreamCreateWithFlags(&e->kabsch_stream, cudaStreamNonBlocking));
+    CUC(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
+    CUC(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
+    CUC(cudaEventCreateWithFlags(&e->ev_fwd, cudaEventDisableTiming));
 #undef CUC
     *out = e;
     return DSAC_OK;
@@ -506,9 +451,8 @@ int64_t dsac_launch_count(const dsac_engine* e) { return e ? e->launches : 0; }
 
 int dsac_sampler_profile(dsac_engine* e, int32_t enable) {
     if (!e) return DSAC_ERR_ARG;
-    if (!e->k1_mode) return fail(e, DSAC_ERR_ARG, "dsac_sampler_profile needs the split sampler (DSAC_K1_MODE unset)");
     CU(cudaSetDevice(e->cfg.device));
-    if (enable && !e->d_k1_dbg) CU(cudaMalloc(&e->d_k1_dbg, K1S_MAX_ROUNDS * 4 * sizeof(unsigned long long)));
+    if (enable && !e->d_k1_dbg) CU(dev_alloc(e, &e->d_k1_dbg, K1S_MAX_ROUNDS * 4 * sizeof(unsigned long long)));
     e->k1_profile = enable ? 1 : 0;
     return DSAC_OK;
 }
@@ -559,7 +503,7 @@ int dsac_set_score_backward_hook(dsac_engine* e, dsac_score_backward_hook fn, vo
     return DSAC_OK;
 }
 
-// Score seam in the backward pass: with hooks registered, dScore/dDiffMap comes from the backward hook (fills e->d_ext_g);
+// Score seam in the backward pass: with hooks registered, dScore/dDiffMap comes from the backward hook (fills e->ext_g);
 // returns the pointer k_dscore shall read (null: closed-form soft-inlier derivative).
 static int seam_backward(dsac_engine* e, int n, const double* d_sog, cudaStream_t stream, const double** ext_g) {
     *ext_g = nullptr;
@@ -569,20 +513,15 @@ static int seam_backward(dsac_engine* e, int n, const double* d_sog, cudaStream_
                     e->hook ? "the forward hook" : "the backward hook", e->hook ? "the backward hook" : "the forward hook");
     if (!e->d_diffmaps) return fail(e, DSAC_ERR_ARG, "the score seam needs write_diffmaps=1");
     const size_t H = e->cfg.n_hyps, count = (size_t)n * H * DSAC_N;
-    if (count > e->ext_g_count) {
-        if (e->d_ext_g) cudaFree(e->d_ext_g);
-    if (e->d_kabsch) cudaFree(e->d_kabsch);
-        e->d_ext_g = nullptr; e->ext_g_count = 0;
-        CU(cudaMalloc(&e->d_ext_g, (count + (size_t)n * H) * sizeof(double)));
-        e->ext_g_count = count;
-    }
-    double* clamped = e->d_ext_g + e->ext_g_count;   // [n][H] behind the gradient block
+    CU(e->ext_g.reserve((count + (size_t)n * H) * sizeof(double)));
+    double* grad = (double*)e->ext_g.ptr;
+    double* clamped = grad + count;   // [n][H] behind the gradient block
     k_clamp_copy<<<(unsigned)(((size_t)n * H + 255) / 256), 256, 0, stream>>>(d_sog, clamped, (size_t)n * H, e->cfg.grad_clamp);
     e->launches++;
     CU(cudaGetLastError());
-    int rc = e->bw_hook(e->d_diffmaps, clamped, n, (int32_t)H, e->d_ext_g, (void*)stream, e->bw_hook_user);
+    int rc = e->bw_hook(e->d_diffmaps, clamped, n, (int32_t)H, grad, (void*)stream, e->bw_hook_user);
     if (rc != 0) return fail(e, DSAC_ERR_ARG, "score backward hook returned %d", rc);
-    *ext_g = e->d_ext_g;
+    *ext_g = grad;
     return DSAC_OK;
 }
 
@@ -598,11 +537,166 @@ static int pick_tile(const dsac_engine* e, int n_frames) {
     return t;
 }
 
-// Launches the forward stages for `n` frames whose per-frame engine buffers start at frame offset `off`
-// (inputs are passed already offset).  Used whole (off = 0) and per chunk by the pipelined host path.
+// The split sampler (sampler_split.cuh) for the `n` frames at frame offset `off`, on lane L: the generator on `stream`, filter
+// and solve on the lane's side streams.  One pass at a time per lane: the queues and per-slot arrays are the engine's,
+// sliced by frame offset.
+static int sample_split(dsac_engine* e, K1Lane& L, int32_t off, int32_t n, SampleParams sp, cudaStream_t stream) {
+    const dsac_config& c = e->cfg;
+    const size_t o = (size_t)off, Nn = DSAC_N, T = (size_t)c.n_streams, cap = (size_t)e->k1_cap;
+    K1SplitParams q;
+    q.sp = sp;
+    q.state = e->d_k1_state + o * T; q.celltab = e->d_k1_celltab + o * Nn;
+    q.cells = e->d_k1_cells + o * T * cap; q.endw = e->d_k1_endw + o * T * cap;
+    q.accbits = e->d_k1_accbits + o * T * (cap / 32); q.pose_out = e->d_k1_pose + o * T * cap * 6;
+    q.wq = e->d_k1_wq + o * T * 128; q.fq = e->d_k1_fq + o * T * cap;   // (work items / flagged candidates of this range's slots)
+    q.wq_n = L.counters; q.fq_n = L.counters + K1S_MAX_SETS;
+    q.wq_stride = e->k1_wq_stride;
+    q.first_frac = (double)K1S_FIRST_ROUND_FRAC;
+    q.spec = 0;
+    const int par = (int)(L.calls & 1ull);
+    L.calls++;
+    q.stats_cur = L.stats + 2 * par; q.stats_prev = L.stats + 2 * (par ^ 1);
+    q.dbg = e->d_k1_dbg;
+    q.cap = e->k1_cap;
+    const long long n_slots = (long long)n * c.n_streams;
+    // a round is generated in up to 4 portions of cap / 4 candidates (round 0: 4, round 1: 2, later rounds: the whole
+    // round at once); a filter work item is a chunk of a portion.  Measured at 128 frames: 2 / 4 / 8 / 16 portions
+    // 0.885 / 0.896 / 0.951 / 1.207 ms per step (1024 frames: 2.94 / 2.89 / 2.97 / -)
+    const int n_port = n_slots < 256 ? 2 : 4;   // portions of round 0 (round 1: half as many, twice as large)
+    const int portion4 = e->k1_cap / n_port;
+    const int want_chunk = n_slots >= 512 ? 2048 : (n_slots >= 64 ? 512 : 256);
+    q.chunk = 256;
+    for (int cc : {2048, 1024, 512, 256})
+        if (cc <= want_chunk && cc <= K1F_MAX_CHUNK && portion4 % cc == 0) { q.chunk = cc; break; }
+    q.n_slots = (int)n_slots;
+    q.round = 0; q.select_only = 0; q.gen_only = 0;
+    CU(cudaMemsetAsync(L.counters, 0, 2 * K1S_MAX_SETS * sizeof(int), stream));
+    CU(cudaMemsetAsync(q.stats_cur, 0, 2 * sizeof(unsigned long long), stream));
+    if (q.dbg) CU(cudaMemsetAsync(q.dbg, 0, K1S_MAX_ROUNDS * 4 * sizeof(unsigned long long), stream));
+    e->k1_ev_n = 0;
+    auto mark = [&](int kind) {   // dsac_sampler_profile: an event after every launch
+        if (!e->k1_profile) return;
+        if ((size_t)e->k1_ev_n >= e->k1_ev.size()) {
+            cudaEvent_t ev;
+            if (cudaEventCreate(&ev) != cudaSuccess) return;
+            e->k1_ev.push_back(ev);
+            e->k1_ev_kind.push_back(0);
+        }
+        e->k1_ev_kind[e->k1_ev_n] = kind;
+        cudaEventRecord(e->k1_ev[e->k1_ev_n++], stream);
+    };
+    // threads per (frame, stream) of the generator.  A stream's generation is a serial chain of windows; with fewer
+    // streams than the SMs hold at 256 threads, larger CTAs shorten the parallel phases of a window (measured, step in
+    // ms at 256 / 512 / 1024 threads: 128 frames 0.931 / 0.922 / 0.934, 512 frames 1.794 / 1.811 / -; one frame
+    // 295 / - / 272 us).  The MT19937 regeneration itself (half of a window) does not scale: 227 words are independent.
+    int slot_threads = K1S_THREADS;
+    if (n_slots <= 32) slot_threads = 1024;
+    else if (n_slots <= 2 * e->sm_count) slot_threads = 512;
+    if (e->k1_slot_threads > 0) slot_threads = e->k1_slot_threads;
+    auto launch_slot = [&](const K1SplitParams& qq) {
+        const dim3 g(c.n_streams, n);
+        if (slot_threads == 1024) k1_slot_t<1024><<<g, 1024, 0, stream>>>(qq);
+        else if (slot_threads == 512) k1_slot_t<512><<<g, 512, 0, stream>>>(qq);
+        else k1_slot<<<g, K1S_THREADS, 0, stream>>>(qq);
+    };
+    // streams: generator on `stream`, filter (and solve) on a side stream; with a batch that does not fill the GPU several
+    // times over the solve gets a stream of its own, so that the filter of set k+1 need not wait for the solve of set k
+    // (measured, ms per step with the solve on the filter's stream / on its own: 128 frames 0.938 / 0.896, 256 frames
+    // 1.21 / 1.18, 512 frames 1.78 / 1.69, 1024 frames 2.92 / 2.96).  With the profile on everything runs on one stream so
+    // that the event intervals are the kernels' own durations.
+    const bool overlap = !e->k1_profile;
+    cudaStream_t side = overlap ? L.side : stream;
+    cudaStream_t solve_side = (overlap && n_slots <= 768) ? L.side2 : side;
+    const size_t n_slots_cap = (size_t)e->cfg.max_frames * c.n_streams * (size_t)e->k1_cap;
+    mark(-1);
+    {
+        const int cell_blocks = (int)(((size_t)n * Nn + 255) / 256), seed_blocks = (int)((n_slots + 31) / 32);
+        k1_cells<<<(unsigned)(cell_blocks + seed_blocks), 256, 0, stream>>>(q, n, seed_blocks);
+    }
+    mark(0);
+    e->launches++;
+    int set = 0;
+    // few streams (single-frame latency): no previous call's shortfall to make up in later rounds -- the first round
+    // takes 115 % of the expected need and one top-up round follows (every round is three dependent launches);
+    // the rare straggler goes to the monolithic kernel
+    const bool few = n_slots < 128;
+    if (few) q.first_frac = 1.15;
+    // speculative first round (k1_spec / k1_stitch): one stream generated window by window on many SMs; pays when a
+    // stream's first round is several windows long (>= 64 hypotheses per stream) and the GPU is otherwise idle
+    const int quota_max = (c.n_hyps + c.n_streams - 1) / c.n_streams;
+    const bool use_spec = few && off == 0 && n_slots <= e->k1_spec_slots && quota_max >= 64 && c.max_candidates >= (1 << 16);   // (the candidate bound cannot fall inside the speculative round)
+    // chained generator (k1_pipe): K CTAs per stream, all of them resident at once
+    const int pipe_K = (int)std::min<long long>(8, e->k1_slot_capacity / std::max<long long>(1, n_slots));
+    const bool use_pipe = e->k1_pipe && !use_spec && pipe_K >= 3 && n_slots >= 9 && quota_max >= 64 && c.max_candidates >= (1 << 16) &&
+                          !e->k1_profile;
+    const int n_rounds = few ? std::min(K1_ROUNDS, 2) : K1_ROUNDS;
+    for (int r = 0; r < n_rounds; r++) {
+        // portions only pay when the generator has the whole GPU to fill (many streams); a few streams (single-frame
+        // latency, BASELINE config 2) take every round in one launch set: fewer dependent launches
+        const bool portioned = n_slots >= 128 && r < 2 && !(use_pipe && r == 0);
+        const int sets = portioned ? (r == 0 ? n_port : n_port / 2) : 1;
+        q.round = r;
+        q.portion = portioned ? (r == 0 ? portion4 : 2 * portion4) : e->k1_cap;   // round 1 may use the whole capacity too
+        q.round_limit = q.portion * sets;
+        const int fgrid = (int)std::min<long long>(e->k1_filter_grid, n_slots * ((q.portion + q.chunk - 1) / q.chunk));
+        if (overlap && r > 0) CU(cudaStreamWaitEvent(stream, L.ev_round, 0));   // the selection needs the previous round's solves
+        for (int k = 0; k < sets && set < K1S_MAX_SETS; k++, set++) {
+            q.gen_only = (k > 0);
+            q.qidx = set;
+            q.fqidx = set;
+            q.fq = e->d_k1_fq + o * T * cap + (size_t)(set & 1) * n_slots_cap;
+            if (use_spec && r == 0 && k == 0) {
+                K1SpecParams spp;
+                spp.vstate = e->d_k1_vstate; spp.vcells = e->d_k1_vcells; spp.vendw = e->d_k1_vendw; spp.result = e->d_k1_spec_result; spp.table = e->d_k1_spec_table;
+                k1_spec<<<dim3(K1P_VPER, (unsigned)n_slots), K1S_THREADS, 0, stream>>>(q, spp);
+                k1_stitch<<<(unsigned)n_slots, K1T_THREADS, 0, stream>>>(q, spp);
+                k1_gather<<<dim3((unsigned)((e->k1_cap + K1G_PER_CTA - 1) / K1G_PER_CTA), (unsigned)n_slots), K1G_THREADS, 0, stream>>>(q, spp);
+                e->launches += 2;
+            } else if (use_pipe && r == 0 && k == 0) {
+                K1PipeParams ppm;
+                ppm.chain = e->d_k1_chain + o * T * (K1Q_MAX_WIN + 1) * 4;
+                ppm.epoch = (uint32_t)(++e->k1_epoch & 0x7fffffffull) + 1u;
+                ppm.K = pipe_K;
+                k1_pipe<<<dim3((unsigned)pipe_K, (unsigned)n_slots), K1S_THREADS, 0, stream>>>(q, ppm);
+            } else {
+                launch_slot(q);
+            }
+            mark(0);
+            if (overlap) {
+                CU(cudaEventRecord(L.ev_gen[set], stream));
+                CU(cudaStreamWaitEvent(side, L.ev_gen[set], 0));
+                if (solve_side != side && set >= 2) CU(cudaStreamWaitEvent(side, L.ev_solve[set - 2], 0));   // the flag-queue region is free again
+            }
+            k1_filter<<<fgrid, K1F_THREADS, sizeof(K1FSmem), side>>>(q);
+            if (!overlap) mark(1);
+            if (solve_side != side) {
+                CU(cudaEventRecord(L.ev_filt[set], side));
+                CU(cudaStreamWaitEvent(solve_side, L.ev_filt[set], 0));
+            }
+            if (few) k1_solve4<<<e->k1_solve_grid, K1V_THREADS, 0, solve_side>>>(q);
+            else k1_solve<<<e->k1_solve_grid, K1V_THREADS, 0, solve_side>>>(q);
+            if (solve_side != side) CU(cudaEventRecord(L.ev_solve[set], solve_side));
+            if (!overlap) mark(2);
+            e->launches += 3;
+        }
+        if (overlap) CU(cudaEventRecord(L.ev_round, solve_side));
+    }
+    if (overlap) CU(cudaStreamWaitEvent(stream, L.ev_round, 0));
+    q.round = n_rounds; q.select_only = 1; q.gen_only = 0;
+    launch_slot(q);
+    mark(0);
+    sp.resume = q.state;   // streams the rounds left unfinished (normally none) continue in the monolithic kernel
+    k_sample<<<dim3(c.n_streams, n), K1_THREADS, sizeof(K1Smem), stream>>>(sp);
+    mark(3);
+    e->launches += 2;
+    CU(cudaGetLastError());
+    return DSAC_OK;
+}
+
+// Launches the forward stages for `n` frames whose per-frame engine buffers start at frame offset `off` (inputs are passed
+// already offset), with the sampler on lane `lane`.  Used whole (off = 0) and per half-batch by forward_split.
 static int forward_range(dsac_engine* e, int32_t off, int32_t n, int64_t frame0, const int16_t* d_coords, const int32_t* d_pix,
-                         int32_t pix_shared, const double* d_gt_jp, void* stream_v, int lane = 0) {
-    cudaStream_t stream = (cudaStream_t)stream_v;
+                         int32_t pix_shared, const double* d_gt_jp, cudaStream_t stream, int lane = 0) {
     const dsac_config& c = e->cfg;
     const size_t o = (size_t)off, Hh = (size_t)c.n_hyps, Nn = DSAC_N;
 
@@ -619,210 +713,8 @@ static int forward_range(dsac_engine* e, int32_t off, int32_t n, int64_t frame0,
         sp.phase_cycles = e->d_phase;
         { const char* g = getenv("DSAC_K1_A2_GENERIC"); sp.a2_generic = (g && g[0] == '1') ? 1 : 0; }
         sp.resume = nullptr;
-        if (!e->k1_mode) {
-            k_sample<<<dim3(c.n_streams, n), K1_THREADS, sizeof(K1Smem), stream>>>(sp);
-            e->launches++;
-            CU(cudaGetLastError());
-        } else {
-            // round-based pipeline (sampler_split.cuh).  One pass at a time per engine: the queues are shared.
-            const size_t T = (size_t)c.n_streams, cap = (size_t)e->k1_cap;
-            // the lane's own streams, events, counters and statistics (lane 0: the engine's; lane 1: e->lane1)
-            cudaStream_t k_side = lane ? e->lane1.side : e->k1_side, k_side2 = lane ? e->lane1.side2 : e->k1_side2;
-            cudaEvent_t* k_ev_filt = lane ? e->lane1.ev_filt : e->k1_ev_filt;
-            cudaEvent_t* k_ev_solve = lane ? e->lane1.ev_solve : e->k1_ev_solve;
-            cudaEvent_t* k_ev_gen = lane ? e->lane1.ev_gen : e->k1_ev_gen;
-            cudaEvent_t k_ev_round = lane ? e->lane1.ev_round : e->k1_ev_round;
-            int* k_counters = lane ? e->lane1.counters : e->d_k1_counters;
-            unsigned long long* k_stats = lane ? e->lane1.stats : e->d_k1_stats;
-            unsigned long long& k_calls = lane ? e->lane1.calls : e->k1_calls;
-            K1SplitParams q;
-            q.sp = sp;
-            q.state = e->d_k1_state + o * T; q.celltab = e->d_k1_celltab + o * Nn;
-            q.cells = e->d_k1_cells + o * T * cap; q.endw = e->d_k1_endw + o * T * cap;
-            q.accbits = e->d_k1_accbits + o * T * (cap / 32); q.pose_out = e->d_k1_pose + o * T * cap * 6;
-            q.wq = e->d_k1_wq + o * T * 128; q.fq = e->d_k1_fq + o * T * cap;   // (work items / flagged candidates of this range's slots)
-            q.wq_n = k_counters; q.fq_n = k_counters + K1S_MAX_SETS;
-            q.wq_stride = e->k1_wq_stride;
-            q.first_frac = (double)K1S_FIRST_ROUND_FRAC;
-            q.spec = 0;
-            const int par = (int)(k_calls & 1ull);
-            k_calls++;
-            q.stats_cur = k_stats + 2 * par; q.stats_prev = k_stats + 2 * (par ^ 1);
-            q.dbg = e->d_k1_dbg;
-            q.cap = e->k1_cap;
-            const long long n_slots = (long long)n * c.n_streams;
-            // a round is generated in up to 4 portions of cap / 4 candidates (round 0: 4, round 1: 2, later rounds: the whole
-            // round at once); a filter work item is a chunk of a portion
-            int n_port = 4;                       // portions of round 0 (round 1: half as many, twice as large)
-            bool port_forced = false;
-            if (const char* pp = getenv("DSAC_K1_PORTIONS")) {
-                const int v = atoi(pp);
-                if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16) { n_port = v; port_forced = true; }
-            }
-            if (!port_forced && n_slots < 256) n_port = 2;   // measured at 128 frames: 2 / 4 / 8 / 16 portions 0.885 / 0.896 / 0.951 / 1.207 ms per step (1024 frames: 2.94 / 2.89 / 2.97 / -)
-            const int portion4 = e->k1_cap / n_port;
-            int want_chunk = n_slots >= 512 ? 2048 : (n_slots >= 64 ? 512 : 256);
-            if (const char* ch = getenv("DSAC_K1_CHUNK")) want_chunk = std::max(256, atoi(ch));
-            q.chunk = 256;
-            for (int cc : {2048, 1024, 512, 256})
-                if (cc <= want_chunk && cc <= K1F_MAX_CHUNK && portion4 % cc == 0) { q.chunk = cc; break; }
-            q.n_slots = (int)n_slots;
-            q.round = 0; q.select_only = 0; q.gen_only = 0;
-            CU(cudaMemsetAsync(k_counters, 0, 2 * K1S_MAX_SETS * sizeof(int), stream));
-            CU(cudaMemsetAsync(q.stats_cur, 0, 2 * sizeof(unsigned long long), stream));
-            if (q.dbg) CU(cudaMemsetAsync(q.dbg, 0, K1S_MAX_ROUNDS * 4 * sizeof(unsigned long long), stream));
-            e->k1_ev_n = 0;
-            auto mark = [&](int kind) {   // dsac_sampler_profile: an event after every launch
-                if (!e->k1_profile) return;
-                if ((size_t)e->k1_ev_n >= e->k1_ev.size()) {
-                    cudaEvent_t ev;
-                    if (cudaEventCreate(&ev) != cudaSuccess) return;
-                    e->k1_ev.push_back(ev);
-                    e->k1_ev_kind.push_back(0);
-                }
-                e->k1_ev_kind[e->k1_ev_n] = kind;
-                cudaEventRecord(e->k1_ev[e->k1_ev_n++], stream);
-            };
-            // threads per (frame, stream) of the generator.  A stream's generation is a serial chain of windows; with fewer
-            // streams than the SMs hold at 256 threads, larger CTAs shorten the parallel phases of a window (measured, step in
-            // ms at 256 / 512 / 1024 threads: 128 frames 0.931 / 0.922 / 0.934, 512 frames 1.794 / 1.811 / -; one frame
-            // 295 / - / 272 us).  The MT19937 regeneration itself (half of a window) does not scale: 227 words are independent.
-            int slot_threads = K1S_THREADS;
-            if (n_slots <= 32) slot_threads = 1024;
-            else if (n_slots <= 2 * e->sm_count) slot_threads = 512;
-            if (e->k1_slot_threads > 0) slot_threads = e->k1_slot_threads;
-            auto launch_slot = [&](const K1SplitParams& qq) {
-                const dim3 g(c.n_streams, n);
-                if (slot_threads == 1024) k1_slot_t<1024><<<g, 1024, 0, stream>>>(qq);
-                else if (slot_threads == 512) k1_slot_t<512><<<g, 512, 0, stream>>>(qq);
-                else k1_slot<<<g, K1S_THREADS, 0, stream>>>(qq);
-            };
-            // with the profile on everything runs on one stream so that the event intervals are the kernels' own durations
-            const bool fused = e->k1_fused != 0;
-            // streams: generator on `stream`, filter (and solve) on a side stream; with a batch that does not fill the GPU several
-            // times over the solve gets a stream of its own, so that the filter of set k+1 need not wait for the solve of set k
-            // (measured, ms per step with the solve on the filter's stream / on its own: 128 frames 0.938 / 0.896, 256 frames
-            // 1.21 / 1.18, 512 frames 1.78 / 1.69, 1024 frames 2.92 / 2.96)
-            const int ov_mode = e->k1_overlap_fixed ? e->k1_overlap : (n_slots <= 768 ? 2 : 1);
-            const bool overlap = ov_mode && !e->k1_profile && !fused;
-            cudaStream_t side = overlap ? k_side : stream;
-            cudaStream_t solve_side = (overlap && ov_mode >= 2) ? k_side2 : side;
-            const size_t n_slots_cap = (size_t)e->cfg.max_frames * c.n_streams * (size_t)e->k1_cap;
-            mark(-1);
-            {
-                const int cell_blocks = (int)(((size_t)n * Nn + 255) / 256), seed_blocks = (int)((n_slots + 31) / 32);
-                k1_cells<<<(unsigned)(cell_blocks + seed_blocks), 256, 0, stream>>>(q, n, seed_blocks);
-            }
-            mark(0);
-            e->launches++;
-            int set = 0;
-            // few streams (single-frame latency): no previous call's shortfall to make up in later rounds -- the first round
-            // takes 115 % of the expected need and one top-up round follows (every round is three dependent launches);
-            // the rare straggler goes to the monolithic kernel
-            const bool few = n_slots < 128;
-            const bool fused_req = e->k1_fused != 0;
-            if (few) q.first_frac = 1.15;
-            // speculative first round (k1_spec / k1_stitch): one stream generated window by window on many SMs; pays when a
-            // stream's first round is several windows long (>= 64 hypotheses per stream) and the GPU is otherwise idle
-            const int quota_max = (c.n_hyps + c.n_streams - 1) / c.n_streams;
-            const bool use_spec = few && off == 0 && n_slots <= e->k1_spec_slots && quota_max >= 64 && c.max_candidates >= (1 << 16) && !fused_req;   // (the candidate bound cannot fall inside the speculative round)
-            // chained generator (k1_pipe): K CTAs per stream, all of them resident at once
-            const int pipe_K = (int)std::min<long long>(8, e->k1_slot_capacity / std::max<long long>(1, n_slots));
-            const bool use_pipe = e->k1_pipe && !use_spec && pipe_K >= 3 && n_slots >= 9 && quota_max >= 64 && c.max_candidates >= (1 << 16) &&
-                                  !fused_req && !e->k1_profile;
-            const int n_rounds = (few && !e->k1_rounds_fixed) ? std::min(e->k1_rounds, 2) : e->k1_rounds;
-            for (int r = 0; r < n_rounds; r++) {
-                // portions only pay when the generator has the whole GPU to fill (many streams); a few streams (single-frame
-                // latency, BASELINE config 2) take every round in one launch set: fewer dependent launches
-                const bool portioned = (n_slots >= 128 || port_forced) && r < 2 && n_port > 1 && !(use_pipe && r == 0);
-                const int sets = portioned ? (r == 0 ? n_port : n_port / 2) : 1;
-                q.round = r;
-                q.portion = portioned ? (r == 0 ? portion4 : 2 * portion4) : e->k1_cap;   // round 1 may use the whole capacity too
-                q.round_limit = q.portion * sets;
-                const int fgrid = (int)std::min<long long>(e->k1_filter_grid, n_slots * ((q.portion + q.chunk - 1) / q.chunk));
-                if (overlap && r > 0) CU(cudaStreamWaitEvent(stream, k_ev_round, 0));   // the selection needs the previous round's solves
-                if (fused) {
-                    // one stream: slot (select + first portion), then per set { filter(k) | generator(k+1) } fused, solve(k)
-                    q.gen_only = 0; q.qidx = set; q.fqidx = set; q.fq = e->d_k1_fq + o * T * cap + (size_t)(set & 1) * n_slots_cap;
-                    launch_slot(q);
-                    mark(0);
-                    e->launches++;
-                    for (int k = 0; k < sets && set < K1S_MAX_SETS; k++, set++) {
-                        K1SplitParams qf = q;
-                        qf.gen_only = 0; qf.qidx = set; qf.fqidx = set; qf.fq = e->d_k1_fq + o * T * cap + (size_t)(set & 1) * n_slots_cap;
-                        if (k + 1 < sets && set + 1 < K1S_MAX_SETS) {
-                            K1SplitParams qg = q;
-                            qg.gen_only = 1; qg.qidx = set + 1; qg.fqidx = set + 1;
-                            k1_fused<<<e->sm_count, K1X_THREADS, sizeof(K1XSmem), stream>>>(qf, qg);
-                        } else {
-                            k1_filter<<<fgrid, K1F_THREADS, sizeof(K1FSmem), stream>>>(qf);
-                        }
-                        mark(1);
-                        k1_solve<<<e->k1_solve_grid, K1V_THREADS, 0, stream>>>(qf);
-                        mark(2);
-                        e->launches += 2;
-                    }
-                    continue;
-                }
-                const int first_set = set;
-                for (int k = 0; k < sets && set < K1S_MAX_SETS; k++, set++) {
-                    // solve_batch: the sets of a round append to ONE flag queue and a single k1_solve runs after the round's
-                    // last filter (a solve over one set is a partial wave bound by the latency of one P3P)
-                    const bool batch = e->k1_solve_batch != 0;
-                    const bool solve_now = !batch || k + 1 == sets || set + 1 == K1S_MAX_SETS;
-                    const int fset = batch ? first_set : set;
-                    q.gen_only = (k > 0);
-                    q.qidx = set;
-                    q.fqidx = fset;
-                    q.fq = e->d_k1_fq + o * T * cap + (size_t)(fset & 1) * (size_t)n_slots_cap;
-                    if (use_spec && r == 0 && k == 0) {
-                        K1SpecParams spp;
-                        spp.vstate = e->d_k1_vstate; spp.vcells = e->d_k1_vcells; spp.vendw = e->d_k1_vendw; spp.result = e->d_k1_spec_result; spp.table = e->d_k1_spec_table;
-                        k1_spec<<<dim3(K1P_VPER, (unsigned)n_slots), K1S_THREADS, 0, stream>>>(q, spp);
-                        k1_stitch<<<(unsigned)n_slots, K1T_THREADS, 0, stream>>>(q, spp);
-                        k1_gather<<<dim3((unsigned)((e->k1_cap + K1G_PER_CTA - 1) / K1G_PER_CTA), (unsigned)n_slots), K1G_THREADS, 0, stream>>>(q, spp);
-                        e->launches += 2;
-                    } else if (use_pipe && r == 0 && k == 0) {
-                        K1PipeParams ppm;
-                        ppm.chain = e->d_k1_chain + o * T * (K1Q_MAX_WIN + 1) * 4;
-                        ppm.epoch = (uint32_t)(++e->k1_epoch & 0x7fffffffull) + 1u;
-                        ppm.K = pipe_K;
-                        k1_pipe<<<dim3((unsigned)pipe_K, (unsigned)n_slots), K1S_THREADS, 0, stream>>>(q, ppm);
-                    } else {
-                        launch_slot(q);
-                    }
-                    mark(0);
-                    if (overlap) {
-                        CU(cudaEventRecord(k_ev_gen[set], stream));
-                        CU(cudaStreamWaitEvent(side, k_ev_gen[set], 0));
-                        if (!batch && solve_side != side && set >= 2) CU(cudaStreamWaitEvent(side, k_ev_solve[set - 2], 0));   // the flag-queue region is free again
-                    }
-                    k1_filter<<<fgrid, K1F_THREADS, sizeof(K1FSmem), side>>>(q);
-                    if (!overlap) mark(1);
-                    e->launches += 2;
-                    if (!solve_now) continue;
-                    if (solve_side != side) {
-                        CU(cudaEventRecord(k_ev_filt[set], side));
-                        CU(cudaStreamWaitEvent(solve_side, k_ev_filt[set], 0));
-                    }
-                    if (few && e->k1_solve_group4) k1_solve4<<<e->k1_solve_grid, K1V_THREADS, 0, solve_side>>>(q);
-                    else k1_solve<<<e->k1_solve_grid, K1V_THREADS, 0, solve_side>>>(q);
-                    if (solve_side != side) CU(cudaEventRecord(k_ev_solve[set], solve_side));
-                    if (!overlap) mark(2);
-                    e->launches++;
-                }
-                if (overlap) CU(cudaEventRecord(k_ev_round, solve_side));
-            }
-            if (overlap) CU(cudaStreamWaitEvent(stream, k_ev_round, 0));
-            q.round = n_rounds; q.select_only = 1; q.gen_only = 0;
-            launch_slot(q);
-            mark(0);
-            sp.resume = q.state;   // streams the rounds left unfinished (normally none) continue in the monolithic kernel
-            k_sample<<<dim3(c.n_streams, n), K1_THREADS, sizeof(K1Smem), stream>>>(sp);
-            mark(3);
-            e->launches += 2;
-            CU(cudaGetLastError());
-        }
+        const int rc = sample_split(e, e->lane[lane], off, n, sp, stream);
+        if (rc != DSAC_OK) return rc;
     }
     if (e->stages & DSAC_STAGE_SCORE) {
         ScoreParams kp;
@@ -846,7 +738,7 @@ static int forward_range(dsac_engine* e, int32_t off, int32_t n, int64_t frame0,
         if (e->hook) {
             // score seam (lua_calls.h:284-300): external scorer on the materialised diffmaps,
             // then only the softmax / soft-argmax tail
-            int rc = e->hook(kp.diffmaps, n, c.n_hyps, kp.scores, stream_v, e->hook_user);
+            int rc = e->hook(kp.diffmaps, n, c.n_hyps, kp.scores, (void*)stream, e->hook_user);
             if (rc != 0) return fail(e, DSAC_ERR_ARG, "score hook returned %d", rc);
             kp.external_scores = 1;
             kp.tiles_per_frame = 1;
@@ -878,50 +770,26 @@ static int forward_range(dsac_engine* e, int32_t off, int32_t n, int64_t frame0,
     return DSAC_OK;
 }
 
-// forward_range over the whole batch, with the tail split: the sampler runs one CTA per (frame, stream) and
-// e->k1_slots CTAs are resident at a time, so a batch is a number of whole waves plus a partial one during which
-// most of every SM idles.  Frames [0, n1) (the whole waves) go to the high-priority side stream, the rest stays on
-// `stream`: the block scheduler dispatches the side stream's sampler CTAs first, its scoring / refinement kernels
-// then run next to the partial wave.  Fork / join with events, so for the caller everything still happens in
-// stream order on `stream`.  Frames are independent (disjoint slices of every engine buffer).
+// forward_range over the whole batch.  With allow_split, a batch of at least 768 frames runs as two lanes: two concurrent
+// half-batches, each a complete pass (sampler, H x N matrix, refinement) over its frames with its own queues, counters and
+// side streams.  The passes de-phase on the GPU -- one half's generator and latency-bound refinement run beside the other
+// half's register-filling filter -- which a single pass, whose kernels depend on each other in sequence, cannot: 2.90 ->
+// 2.69 ms per 1024 frames; three or more lanes are slower (3.10 / 3.31 ms: tools/lane_probe.py).  Frames are independent
+// (disjoint slices of every engine buffer) and sampler streams keyed by the global frame index, so results do not depend on
+// the split.  Fork / join with events: for the caller everything still happens in stream order on `stream`.
 static int forward_split(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* d_coords, const int32_t* d_pix,
                          int32_t pix_shared, const double* d_gt_jp, cudaStream_t stream, bool allow_split) {
-    int32_t n1 = 0;
-    if (allow_split && e->tail_split && !e->k1_mode && (e->stages & DSAC_STAGE_SAMPLE) && (e->stages & ~DSAC_STAGE_SAMPLE) && !e->hook) {
-        const int per_wave = e->k1_slots / std::max(1, e->cfg.n_streams);   // frames per sampler wave
-        if (per_wave >= 1 && n > per_wave && n % per_wave != 0) n1 = (n / per_wave) * per_wave;
-    }
-    // Two lanes (split sampler): a large batch as two concurrent half-batches, each a complete pass (sampler, H x N matrix,
-    // refinement) over its frames with its own queues, counters and side streams.  The passes de-phase on the GPU -- one half's
-    // generator and latency-bound refinement run beside the other half's register-filling filter -- which a single pass,
-    // whose kernels depend on each other in sequence, cannot: 2.90 -> 2.69 ms per 1024 frames; three or more lanes are slower
-    // (3.10 / 3.31 ms: tools/lane_probe.py).  Frames are independent and sampler streams keyed by the global frame index, so
-    // results do not depend on the split.
-    if (allow_split && e->k1_mode && e->k1_lanes && n >= 768 && e->lane1.main && !e->k1_profile && !e->d_k1_dbg && !e->k1_fused &&
-        !e->hook && (e->stages & DSAC_STAGE_SAMPLE)) {
-        int32_t na = n / 2;
-        if (const char* lf = getenv("DSAC_K1_LANE_FRAC")) na = std::max(1, std::min(n - 1, (int32_t)(atof(lf) * n)));   // development aid
-        const size_t N = DSAC_N, f = (size_t)na;
-        CU(cudaEventRecord(e->ev_fork, stream));
-        CU(cudaStreamWaitEvent(e->lane1.main, e->ev_fork, 0));
-        int rc = forward_range(e, na, n - na, frame0 + na, d_coords + f * N * 3, pix_shared ? d_pix : d_pix + f * N * 2, pix_shared,
-                               d_gt_jp ? d_gt_jp + f * 12 : nullptr, e->lane1.main, 1);
-        cudaEventRecord(e->ev_join, e->lane1.main);   // the caller's stream joins the lane again whatever happens below
-        if (rc == DSAC_OK) rc = forward_range(e, 0, na, frame0, d_coords, d_pix, pix_shared, d_gt_jp, stream, 0);
-        CU(cudaStreamWaitEvent(stream, e->ev_join, 0));
-        return rc;
-    }
-    if (n1 <= 0) return forward_range(e, 0, n, frame0, d_coords, d_pix, pix_shared, d_gt_jp, stream);
-    const size_t N = DSAC_N, f = (size_t)n1;
+    if (!allow_split || n < 768 || e->k1_profile || e->d_k1_dbg || e->hook || !(e->stages & DSAC_STAGE_SAMPLE))
+        return forward_range(e, 0, n, frame0, d_coords, d_pix, pix_shared, d_gt_jp, stream);
+    const int32_t na = n / 2;
+    const size_t N = DSAC_N, f = (size_t)na;
+    cudaStream_t main1 = e->lane[1].main;
     CU(cudaEventRecord(e->ev_fork, stream));
-    CU(cudaStreamWaitEvent(e->hi, e->ev_fork, 0));
-    int rc = forward_range(e, 0, n1, frame0, d_coords, d_pix, pix_shared, d_gt_jp, e->hi);
-    // whatever happens below, the caller's stream joins the side stream again: nothing may still be writing engine
-    // buffers on e->hi when the caller sees this call's work as complete (or its error)
-    cudaEventRecord(e->ev_join, e->hi);
-    if (rc == DSAC_OK)
-        rc = forward_range(e, n1, n - n1, frame0 + n1, d_coords + f * N * 3, pix_shared ? d_pix : d_pix + f * N * 2, pix_shared,
-                           d_gt_jp ? d_gt_jp + f * 12 : nullptr, stream);
+    CU(cudaStreamWaitEvent(main1, e->ev_fork, 0));
+    int rc = forward_range(e, na, n - na, frame0 + na, d_coords + f * N * 3, pix_shared ? d_pix : d_pix + f * N * 2, pix_shared,
+                           d_gt_jp ? d_gt_jp + f * 12 : nullptr, main1, 1);
+    cudaEventRecord(e->ev_join, main1);   // the caller's stream joins the lane again whatever happens below
+    if (rc == DSAC_OK) rc = forward_range(e, 0, na, frame0, d_coords, d_pix, pix_shared, d_gt_jp, stream, 0);
     CU(cudaStreamWaitEvent(stream, e->ev_join, 0));
     return rc;
 }
@@ -939,8 +807,8 @@ int dsac_forward_device(dsac_engine* e, int32_t n, int64_t frame0, const int16_t
     e->cur_n = n;
     e->dsac_n = 0;
     e->cur_frame0 = frame0;
-    if (e->pending_chunks) return fail(e, DSAC_ERR_ARG, "dsac_forward_device: a submitted pass has not been awaited (dsac_forward_wait)");
-    int rc = forward_split(e, n, frame0, d_coords, d_pix, pix_shared, d_gt_jp, (cudaStream_t)stream_v, true);
+    if (e->pending) return fail(e, DSAC_ERR_ARG, "dsac_forward_device: a submitted pass has not been awaited (dsac_forward_wait)");
+    int rc = forward_split(e, n, frame0, d_coords, d_pix, pix_shared, d_gt_jp, (cudaStream_t)stream_v, e->tail_split >= 1);
     if (rc != DSAC_OK) return rc;
     CU(cudaEventRecord(e->ev_fwd, (cudaStream_t)stream_v));   // dsac_backward (engine stream) waits on this
     return DSAC_OK;
@@ -1019,7 +887,7 @@ int dsac_device_view_get(dsac_engine* e, dsac_device_view* v) {
 static int forward_submit_impl(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* coords, const int32_t* pix,
                                int32_t pix_shared, const double* gt_jp, dsac_forward_out* out, bool blocking) {
     if (!e) return DSAC_ERR_ARG;
-    if (e->pending_chunks) return fail(e, DSAC_ERR_ARG, "dsac_forward_submit: the previous submitted pass has not been awaited");
+    if (e->pending) return fail(e, DSAC_ERR_ARG, "dsac_forward_submit: the previous submitted pass has not been awaited");
     if (n < 1 || n > e->cfg.max_frames) return fail(e, DSAC_ERR_CAPACITY, "n_frames %d exceeds engine capacity %d", n, e->cfg.max_frames);
     if (!coords || !pix) return fail(e, DSAC_ERR_ARG, "null input");
     CU(cudaSetDevice(e->cfg.device));
@@ -1031,63 +899,34 @@ static int forward_submit_impl(dsac_engine* e, int32_t n, int64_t frame0, const 
     e->cur_n = n;
     e->dsac_n = 0;
     e->cur_frame0 = frame0;
-    // Frames are independent, so the batch is cut into up to 4 chunks, each on its own stream:
-    // H2D(chunk) -> K1 -> K2 -> K4 -> D2H(chunk).  Copies of later chunks overlap the kernels of earlier
-    // ones and the tail of one chunk's kernels is filled by the next chunk's CTAs.
+    cudaStream_t st = e->stream;
     static const bool trace = getenv("DSAC_TRACE") != nullptr;
     cudaEvent_t tev[4];
     const auto t_host0 = std::chrono::steady_clock::now();
     if (trace) for (int k = 0; k < 4; k++) cudaEventCreate(&tev[k]);
-    int chunks = 1;   // measured on B200 (tools/e2e_probe.py): 1 chunk 6.03 ms, 2: 6.21, 4: 6.87 -- the sampler kernel wants the whole batch
-    if (const char* ev = getenv("DSAC_PIPE_CHUNKS")) chunks = std::max(1, std::min(4, atoi(ev)));
-    if (pix_shared) CU(cudaMemcpyAsync(e->d_pix, pix, N * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, e->pipe[0]));
-    if (pix_shared && chunks > 1) {   // every chunk reads the shared grid: make it visible to all streams first
-        CU(cudaStreamSynchronize(e->pipe[0]));
+    if (pix_shared) CU(cudaMemcpyAsync(e->d_pix, pix, N * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (trace) cudaEventRecord(tev[0], st);
+    CU(cudaMemcpyAsync(e->d_coords, coords, (size_t)n * N * 3 * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+    if (!pix_shared) CU(cudaMemcpyAsync(e->d_pix, pix, (size_t)n * N * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    if (gt_jp) CU(cudaMemcpyAsync(e->d_gt, gt_jp, (size_t)n * 12 * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (trace) cudaEventRecord(tev[1], st);
+    // two lanes (forward_split) for blocking calls in mode 1: with several submitted passes in flight the other pass already
+    // fills the GPU; mode 2: always
+    int rc = forward_split(e, n, frame0, e->d_coords, e->d_pix, pix_shared, gt_jp ? e->d_gt : nullptr, st,
+                           blocking ? e->tail_split >= 1 : e->tail_split >= 2);
+    if (trace) cudaEventRecord(tev[2], st);
+    if (rc == DSAC_OK && out) rc = fetch_range(e, 0, n, out, st);
+    if (rc != DSAC_OK) {   // copies from the caller's host buffers may already be queued: drain before reporting
+        cudaStreamSynchronize(st);
+        return rc;
     }
-    // chunk boundaries at whole waves of the sampler (one CTA per frame and stream, e->k1_slots CTAs resident per GPU),
-    // so that a later chunk's CTAs fill the slots an earlier chunk frees instead of adding a partial wave
-    int bound[5] = {0, n, n, n, n};
-    if (chunks > 1) {
-        const int per_wave = std::max(1, e->k1_slots / std::max(1, e->cfg.n_streams));
-        const int waves = (n + per_wave - 1) / per_wave;
-        for (int c = 1; c < chunks; c++) bound[c] = std::min(n, std::max(1, (int)((long long)waves * c / chunks)) * per_wave);
-        bound[chunks] = n;
-    }
-    for (int c = 0; c < chunks; c++) {
-        const int lo = bound[c], hi = bound[c + 1], m = hi - lo;
-        if (m <= 0) continue;
-        cudaStream_t st = e->pipe[c];
-        const size_t f = (size_t)lo;
-        if (trace) cudaEventRecord(tev[0], st);
-        CU(cudaMemcpyAsync(e->d_coords + f * N * 3, coords + f * N * 3, (size_t)m * N * 3 * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-        if (!pix_shared)
-            CU(cudaMemcpyAsync(e->d_pix + f * N * 2, pix + f * N * 2, (size_t)m * N * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        if (gt_jp) CU(cudaMemcpyAsync(e->d_gt + f * 12, gt_jp + f * 12, (size_t)m * 12 * sizeof(double), cudaMemcpyHostToDevice, st));
-        if (trace) cudaEventRecord(tev[1], st);
-        // one chunk: the tail split applies (mode 1: blocking calls only -- with several passes in flight the other
-        // pass already fills the partial wave and a high-priority stream would only delay it; mode 2: always)
-        int rc = (chunks == 1)
-                     ? forward_split(e, m, frame0, e->d_coords, e->d_pix, pix_shared, gt_jp ? e->d_gt : nullptr, st,
-                                     blocking ? e->tail_split >= 1 : e->tail_split >= 2)
-                     : forward_range(e, lo, m, frame0 + lo, e->d_coords + f * N * 3, pix_shared ? e->d_pix : e->d_pix + f * N * 2,
-                                     pix_shared, gt_jp ? e->d_gt + f * 12 : nullptr, st);
-        if (rc == DSAC_OK && out) {
-            if (trace) cudaEventRecord(tev[2], st);
-            rc = fetch_range(e, lo, m, out, st);
-        }
-        if (rc != DSAC_OK) {   // copies from the caller's host buffers may already be queued: drain before reporting
-            for (int k = 0; k <= c; k++) cudaStreamSynchronize(e->pipe[k]);
-            return rc;
-        }
-        if (trace && !out) cudaEventRecord(tev[2], st);
-        if (trace) cudaEventRecord(tev[3], st);
-    }
+    if (trace) cudaEventRecord(tev[3], st);
     e->pending_out = out;
     e->pending_n = n;
-    e->pending_chunks = chunks;
-    CU(cudaEventRecord(e->ev_fwd, e->pipe[chunks - 1]));
-    if (trace) {   // DSAC_TRACE=1: where one pass spends its time (last chunk's stream); forces the wait
-        for (int c = 0; c < chunks; c++) CU(cudaStreamSynchronize(e->pipe[c]));
+    e->pending = true;
+    CU(cudaEventRecord(e->ev_fwd, st));
+    if (trace) {   // DSAC_TRACE=1: where one pass spends its time; forces the wait
+        CU(cudaStreamSynchronize(st));
         float a = 0, b = 0, d = 0;
         cudaEventElapsedTime(&a, tev[0], tev[1]); cudaEventElapsedTime(&b, tev[1], tev[2]); cudaEventElapsedTime(&d, tev[2], tev[3]);
         const double host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count();
@@ -1099,11 +938,10 @@ static int forward_submit_impl(dsac_engine* e, int32_t n, int64_t frame0, const 
 
 int dsac_forward_wait(dsac_engine* e) {
     if (!e) return DSAC_ERR_ARG;
-    if (!e->pending_chunks) return DSAC_OK;
+    if (!e->pending) return DSAC_OK;
     CU(cudaSetDevice(e->cfg.device));
-    const int chunks = e->pending_chunks;
-    e->pending_chunks = 0;
-    for (int c = 0; c < chunks; c++) CU(cudaStreamSynchronize(e->pipe[c]));
+    e->pending = false;
+    CU(cudaStreamSynchronize(e->stream));
     if (e->pending_out) sum_candidates(e, e->pending_n, e->pending_out);
     e->pending_out = nullptr;
     return DSAC_OK;
@@ -1124,40 +962,34 @@ int dsac_forward(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* coord
 int dsac_forward_dsac(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* coords, const int32_t* pix,
                       int32_t pix_shared, const double* gt_jp, int32_t random_draw, dsac_dsac_out* out) {
     if (!e || !out) return DSAC_ERR_ARG;
-    if (e->pending_chunks) return fail(e, DSAC_ERR_ARG, "dsac_forward_dsac: a submitted pass has not been awaited (dsac_forward_wait)");
+    if (e->pending) return fail(e, DSAC_ERR_ARG, "dsac_forward_dsac: a submitted pass has not been awaited (dsac_forward_wait)");
     if (n < 1 || n > e->cfg.max_frames) return fail(e, DSAC_ERR_CAPACITY, "n_frames %d exceeds engine capacity %d", n, e->cfg.max_frames);
     if (!coords || !pix) return fail(e, DSAC_ERR_ARG, "null input");
     const dsac_config& c = e->cfg;
     CU(cudaSetDevice(c.device));
-    cudaStream_t stream = e->pipe[0];
+    cudaStream_t stream = e->stream;
     const size_t N = DSAC_N, nn = (size_t)n, H = c.n_hyps, jobs = nn * H, T = c.n_streams;
-    // refine-all buffers
+    // refine-all buffers: one block, carved for ra_jobs jobs; the job -> frame table is written when it grows
     if (jobs > e->ra_jobs) {
-        void* old[] = {e->d_ra_frame, e->d_ra_pose, e->d_ra_loss, e->d_ra_rot, e->d_ra_t, e->d_ra_correct, e->d_ra_steps};
-        for (void* q : old)
-            if (q) cudaFree(q);
-        e->d_ra_frame = nullptr; e->d_ra_pose = nullptr; e->d_ra_loss = nullptr; e->d_ra_rot = nullptr; e->d_ra_t = nullptr;
-        e->d_ra_correct = nullptr; e->d_ra_steps = nullptr;
         e->ra_jobs = 0;
-        CU(cudaMalloc(&e->d_ra_frame, jobs * sizeof(int32_t)));
-        CU(cudaMalloc(&e->d_ra_pose, jobs * 6 * sizeof(double)));
-        CU(cudaMalloc(&e->d_ra_loss, jobs * sizeof(double)));
-        CU(cudaMalloc(&e->d_ra_rot, jobs * sizeof(double)));
-        CU(cudaMalloc(&e->d_ra_t, jobs * sizeof(double)));
-        CU(cudaMalloc(&e->d_ra_correct, jobs * sizeof(int32_t)));
-        CU(cudaMalloc(&e->d_ra_steps, jobs * sizeof(int32_t)));
+        auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const size_t b6 = al(jobs * 6 * sizeof(double)), bd = al(jobs * sizeof(double)), bi = al(jobs * sizeof(int32_t));
+        CU(e->ra.reserve(b6 + 3 * bd + 3 * bi));
+        char* p = (char*)e->ra.ptr;
+        e->d_ra_pose = (double*)p; p += b6;
+        e->d_ra_loss = (double*)p; p += bd;
+        e->d_ra_rot = (double*)p; p += bd;
+        e->d_ra_t = (double*)p; p += bd;
+        e->d_ra_frame = (int32_t*)p; p += bi;
+        e->d_ra_correct = (int32_t*)p; p += bi;
+        e->d_ra_steps = (int32_t*)p;
         std::vector<int32_t> jf(jobs);
         for (size_t j = 0; j < jobs; j++) jf[j] = (int32_t)(j / H);
         CU(cudaMemcpy(e->d_ra_frame, jf.data(), jobs * sizeof(int32_t), cudaMemcpyHostToDevice));
         e->ra_jobs = jobs;
     }
-    if (out->inlier_maps && jobs > e->ra_imap_jobs) {
-        if (e->d_ra_imap) cudaFree(e->d_ra_imap);
-        e->d_ra_imap = nullptr;
-        e->ra_imap_jobs = 0;
-        CU(cudaMalloc(&e->d_ra_imap, jobs * N * sizeof(int32_t)));
-        e->ra_imap_jobs = jobs;
-    }
+    if (out->inlier_maps) CU(e->ra_imap.reserve(jobs * N * sizeof(int32_t)));
+    int32_t* d_ra_imap = out->inlier_maps ? (int32_t*)e->ra_imap.ptr : nullptr;
     CU(cudaMemcpyAsync(e->d_coords, coords, nn * N * 3 * sizeof(int16_t), cudaMemcpyHostToDevice, stream));
     CU(cudaMemcpyAsync(e->d_pix, pix, (pix_shared ? 1 : nn) * N * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
     if (gt_jp) CU(cudaMemcpyAsync(e->d_gt, gt_jp, nn * 12 * sizeof(double), cudaMemcpyHostToDevice, stream));
@@ -1182,7 +1014,7 @@ int dsac_forward_dsac(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* 
         rp.job_init = e->d_hyp_pose;
         rp.out_pose = e->d_ra_pose;
         rp.steps_done = e->d_ra_steps;
-        rp.inlier_map = out->inlier_maps ? e->d_ra_imap : nullptr;
+        rp.inlier_map = d_ra_imap;
         if (e->cur_gt) {
             rp.gt_jp = e->cur_gt;
             rp.loss = e->d_ra_loss; rp.rot_err = e->d_ra_rot; rp.t_err = e->d_ra_t; rp.correct = e->d_ra_correct;
@@ -1211,7 +1043,7 @@ int dsac_forward_dsac(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* 
     D2H(out->entropy, e->d_entropy, nn * sizeof(double));
     D2H(out->ref_pose, e->d_ra_pose, jobs * 6 * sizeof(double));
     D2H(out->steps_done, e->d_ra_steps, jobs * sizeof(int32_t));
-    D2H(out->inlier_maps, e->d_ra_imap, jobs * N * sizeof(int32_t));
+    D2H(out->inlier_maps, d_ra_imap, jobs * N * sizeof(int32_t));
     D2H(out->status, e->d_status, nn * sizeof(uint32_t));
 #undef D2H
     CU(cudaStreamSynchronize(stream));
@@ -1268,13 +1100,13 @@ int dsac_forward_dsac(dsac_engine* e, int32_t n, int64_t frame0, const int16_t* 
 int dsac_backward(dsac_engine* e, int32_t n, const int16_t* coords, const int32_t* pix, int32_t pix_shared,
                   const double* gt_jp, dsac_backward_out* out) {
     if (!e || !out) return DSAC_ERR_ARG;
-    if (e->pending_chunks) return fail(e, DSAC_ERR_ARG, "dsac_backward: a submitted pass has not been awaited (dsac_forward_wait)");
+    if (e->pending) return fail(e, DSAC_ERR_ARG, "dsac_backward: a submitted pass has not been awaited (dsac_forward_wait)");
     return backward_run(e, n, coords, pix, pix_shared, gt_jp, out);
 }
 
 int dsac_backward_dsac(dsac_engine* e, int32_t n, dsac_backward_dsac_out* out) {
     if (!e || !out) return DSAC_ERR_ARG;
-    if (e->pending_chunks) return fail(e, DSAC_ERR_ARG, "dsac_backward_dsac: a submitted pass has not been awaited (dsac_forward_wait)");
+    if (e->pending) return fail(e, DSAC_ERR_ARG, "dsac_backward_dsac: a submitted pass has not been awaited (dsac_forward_wait)");
     return backward_dsac_run(e, n, out);
 }
 

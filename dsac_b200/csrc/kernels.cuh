@@ -19,27 +19,7 @@ namespace dsac {
 // ------------------------------------------------------------------ block helpers
 // Exclusive prefix sum over a block of NWARPS warps (+ block total).  One barrier: consecutive calls must
 // use different s_warp buffers.
-// Barrier over a whole CTA (BAR_ID = 0: __syncthreads) or over a group of BAR_N threads of a warp-specialised CTA (named
-// barrier BAR_ID >= 1: the generator group and the filter group of k1_fused synchronise independently of each other).
-template <int BAR_ID, int BAR_N>
-__device__ __forceinline__ void group_barrier() {
-    if (BAR_ID == 0) __syncthreads();
-    else asm volatile("bar.sync %0, %1;" ::"n"(BAR_ID), "n"(BAR_N) : "memory");
-}
-// barrier + OR of a predicate over the group; flag: a shared int of the group's own
-template <int BAR_ID, int BAR_N>
-__device__ __forceinline__ int group_barrier_or(int pred, int* flag, int tid) {
-    if (BAR_ID == 0) return __syncthreads_or(pred);
-    if (tid == 0) *flag = 0;
-    group_barrier<BAR_ID, BAR_N>();
-    if (pred) *flag = 1;
-    group_barrier<BAR_ID, BAR_N>();
-    const int r = *flag;
-    group_barrier<BAR_ID, BAR_N>();
-    return r;
-}
-
-template <int NWARPS, int BAR_ID = 0, int BAR_N = 0>
+template <int NWARPS>
 __device__ __forceinline__ int block_excl_scan(int v, int* total, int* s_warp /* >= NWARPS ints */, int tid = -1) {
     if (tid < 0) tid = threadIdx.x;
     const int lane = tid & 31, warp = tid >> 5;
@@ -50,7 +30,7 @@ __device__ __forceinline__ int block_excl_scan(int v, int* total, int* s_warp /*
         if (lane >= off) incl += n;
     }
     if (lane == 31) s_warp[warp] = incl;   // callers alternate between two s_warp buffers
-    group_barrier<BAR_ID, BAR_N>();
+    __syncthreads();
     int base = 0, tot = 0;
 #pragma unroll
     for (int w = 0; w < NWARPS; w++) {

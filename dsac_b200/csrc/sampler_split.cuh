@@ -156,7 +156,6 @@ struct K1GSmemT {
     unsigned short brk_ci[K1_BRK_CAP], brk_cur[K1_BRK_CAP];
     int brk_n;
     int sel_total;
-    int or_flag;
 };
 using K1GSmem = K1GSmemT<K1S_WARPS>;
 
@@ -184,11 +183,10 @@ __device__ __forceinline__ int k1_round_size(int quota, int acc, long long cand_
     return r;
 }
 
-// The work of k1_slot for one (frame, stream), by a group of K1S_THREADS threads that synchronise with barrier BAR_ID
-// (0: the whole CTA of the k1_slot kernel; >= 1: the generator warps inside k1_fused).  tid: index within the group.
+// The work of k1_slot for one (frame, stream), by a CTA of NT threads.  tid: thread index.
 // TW3: regeneration through mt_twist3 (own words in registers, branch-free: fastest for a lone CTA -- 230 against 388 cycles per
 // block -- but ten instructions more per thread, which costs the issue-bound full batch 0.05 ms per step)
-template <int BAR_ID, int BAR_N, int NT, bool TW3 = (NT > 256)>
+template <int NT, bool TW3 = (NT > 256)>
 __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT / 32>& sm, const int tid, const int s, const int frame,
                                              const int slot_ov = -1) {
     constexpr int NW = NT / 32, SEL_WORDS = K1S_MAX_CAP / 32 / NT;   // warps of the group; accept-bit words per thread in the selection
@@ -222,7 +220,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
             for (int k = tid; k < ln; k += NT) sm.vals[k] = S.left[k];
             if (tid == 0) { sm.any_reject = S.any_reject; sm.walk_fail = 0; }
         }
-        group_barrier<BAR_ID, BAR_N>();
+        __syncthreads();
     } else if (q.round == 0) {
         if (quota == 0) {
             if (tid == 0) {
@@ -239,7 +237,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
         acc = 0;
         cand_base = 0;
         if (tid == 0) { sm.any_reject = 0; sm.walk_fail = 0; }
-        group_barrier<BAR_ID, BAR_N>();
+        __syncthreads();
     } else {
         if (S.done) return;
         // ---------------- selection: the first (quota - acc) accepted candidates of the previous round, in order
@@ -257,7 +255,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
             mine += __popc(w[k]);
         }
         int tot;
-        int rank = block_excl_scan<NW, BAR_ID, BAR_N>(mine, &tot, sm.warp[0], tid);
+        int rank = block_excl_scan<NW>(mine, &tot, sm.warp[0], tid);
         const int room = quota - acc;
 #pragma unroll
         for (int k = 0; k < SEL_WORDS; k++) {
@@ -270,7 +268,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 rank++;
             }
         }
-        group_barrier<BAR_ID, BAR_N>();
+        __syncthreads();
         const int n_emit = min(tot, room);
         for (int k = tid; k < n_emit; k += NT) {
             const int i = sm.acc_list[k];
@@ -320,7 +318,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
             for (int k = tid; k < ln; k += NT) sm.vals[k] = S.left[k];
             if (tid == 0) { sm.any_reject = S.any_reject; sm.walk_fail = 0; }
         }
-        group_barrier<BAR_ID, BAR_N>();
+        __syncthreads();
     }
 
     // the thread's own three words of the current state, carried in registers from one regeneration to the next (mt_twist3)
@@ -394,7 +392,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 if (rej_any) sm.any_reject = 1;
             }
             gen += MT_N;
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
         }
         K1S_PHASE(0);   // regeneration + decode
         const int w_avail = min((int)(gen - pos), K1S_WORDS);
@@ -464,7 +462,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 }
             }
             if (lane == 0 && warp_id < NWS) sm.ev_n[warp_id] = cnt;
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
             K1S_PHASE(1);   // scan for repeated pairs
             if (tid == 0) {
                 int cur = 0, ci = 0, nb = 1, stop_at = -1;
@@ -496,7 +494,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 sm.brk_n = nb;
                 sm.walk_fail = fail ? 1 : 0;
             }
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
             K1S_PHASE(2);   // thread 0's walk over the events
             if (!sm.walk_fail) {
                 const int n_ok = sm.n_sr, nb = sm.brk_n;
@@ -516,7 +514,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 int extra = 0, start = 0, qn = 0;
                 for (;;) {
                     int tot;
-                    const int excl = block_excl_scan<NW, BAR_ID, BAR_N>(extra, &tot, sm.warp[par], tid);
+                    const int excl = block_excl_scan<NW>(extra, &tot, sm.warp[par], tid);
                     par ^= 1;
                     start = rp + 8 * tid + excl;
                     int cells[4];
@@ -524,20 +522,20 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                     const int ne = (qn < 0) ? 0 : (qn - start) - 8;
                     const int changed = (ne != extra);
                     extra = ne;
-                    if (!group_barrier_or<BAR_ID, BAR_N>(changed, &sm.or_flag, tid)) break;
+                    if (!__syncthreads_or(changed)) break;
                 }
                 int bad = (tid < n_chunk && qn < 0) ? tid : NT;
 #pragma unroll
                 for (int off = 16; off; off >>= 1) bad = min(bad, __shfl_xor_sync(0xffffffffu, bad, off));
                 if (lane == 0) sm.warp[par][tid >> 5] = bad;
-                group_barrier<BAR_ID, BAR_N>();
+                __syncthreads();
                 int n_ok = n_chunk;
 #pragma unroll
                 for (int w = 0; w < NW; w++) n_ok = min(n_ok, sm.warp[par][w]);
                 par ^= 1;
                 if (tid < n_ok) sm.cand_start[n_done + tid] = (unsigned short)start;
                 if (tid == n_ok - 1) sm.newpos = (uint32_t)qn;          // end of the last complete candidate
-                group_barrier<BAR_ID, BAR_N>();
+                __syncthreads();
                 if (n_ok > 0) rp = (int)sm.newpos;
                 n_done += n_ok;
                 out_of_words = (n_ok < n_chunk);
@@ -547,7 +545,7 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 sm.n_sr = n_done;
             }
         }
-        group_barrier<BAR_ID, BAR_N>();
+        __syncthreads();
         K1S_PHASE(3);   // candidate start offsets
         const int n_sr = sm.n_sr;
 
@@ -565,13 +563,13 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
             const int consumed = sm.cand_start[n_sr];
             const int left = w_avail - consumed;
             unsigned char keep[K1S_LEFT_CAP / NT];
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
 #pragma unroll
             for (int k = 0; k < K1S_LEFT_CAP / NT; k++) {
                 const int i = tid + k * NT;
                 keep[k] = (i < left) ? sm.vals[consumed + i] : (unsigned char)0;
             }
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
             bool rej_left = false;
 #pragma unroll
             for (int k = 0; k < K1S_LEFT_CAP / NT; k++) {
@@ -582,12 +580,12 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
                 }
             }
             if (tid == 0) { sm.any_reject = 0; sm.walk_fail = 0; }
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
             if (rej_left) sm.any_reject = 1;   // a rejected draw carried over into the next window
             if (left > K1S_LEFT_CAP && tid == 0) S.overflow = 1;
             pos += (uint32_t)consumed;
             produced += n_sr;
-            group_barrier<BAR_ID, BAR_N>();
+            __syncthreads();
         }
         K1S_PHASE(5);   // leftover move
         if (n_sr == 0) break;   // (cannot happen: every window holds at least one candidate)
@@ -636,11 +634,11 @@ __device__ __forceinline__ void k1_slot_body(const K1SplitParams& q, K1GSmemT<NT
 template <int NT>
 __global__ void __launch_bounds__(NT, (NT == K1S_THREADS) ? K1S_MIN_BLOCKS : 1024 / NT) k1_slot_t(K1SplitParams q) {
     __shared__ K1GSmemT<NT / 32> sm;
-    k1_slot_body<0, 0, NT>(q, sm, threadIdx.x, blockIdx.x, blockIdx.y);
+    k1_slot_body<NT>(q, sm, threadIdx.x, blockIdx.x, blockIdx.y);
 }
 __global__ void __launch_bounds__(K1S_THREADS, K1S_MIN_BLOCKS) k1_slot(K1SplitParams q) {
     __shared__ K1GSmem sm;
-    k1_slot_body<0, 0, K1S_THREADS>(q, sm, threadIdx.x, blockIdx.x, blockIdx.y);
+    k1_slot_body<K1S_THREADS>(q, sm, threadIdx.x, blockIdx.x, blockIdx.y);
 }
 
 // ------------------------------------------------------------------ k1_spec / k1_stitch: one stream generated by many CTAs
@@ -735,7 +733,7 @@ __global__ void __launch_bounds__(K1S_THREADS, K1S_MIN_BLOCKS) k1_spec(K1SplitPa
     K1SplitParams qq = q;
     qq.state = sp.vstate; qq.cells = sp.vcells; qq.endw = sp.vendw; qq.cap = K1P_CAPW;
     qq.round = 1; qq.gen_only = 0; qq.select_only = 0; qq.portion = K1P_NW; qq.round_limit = K1P_NW; qq.spec = 1; qq.dbg = nullptr;
-    k1_slot_body<0, 0, K1S_THREADS, true>(qq, sm, tid, s, frame, vs);
+    k1_slot_body<K1S_THREADS, true>(qq, sm, tid, s, frame, vs);
 }
 
 struct K1StitchSmem {
@@ -1218,7 +1216,7 @@ __device__ __forceinline__ bool k1_filter_candidate(const CellRec* cell, const i
 #endif
 struct K1FSmem {
     CellRec cell[2][DSAC_N_CONST];            // the frame's cell table, double-buffered: 2 x 38.4 KB
-    unsigned short wlist[12][K1F_MAX_CHUNK / 8];   // per warp (8 in k1_filter, 12 in k1_fused): flagged candidates of its share of the item
+    unsigned short wlist[12][K1F_MAX_CHUNK / 8];   // per warp: flagged candidates of its share of the item (8 used; 12 keeps the measured layout)
     unsigned long long mbar[2];               // one transaction barrier per buffer
 };
 
@@ -1229,9 +1227,9 @@ struct K1FSmem {
 // warps run independently: a warp filters every (NTHREADS/32)-th group of 32 candidates of the item (coalesced 8-byte
 // loads of the cell indices, the next group's prefetched), keeps the flagged ones in its own list and appends them to
 // the global queue with one atomic per item.  A group barrier only when moving on to another frame's table.
-// The group: NTHREADS threads synchronising with barrier BAR_ID (0: the whole CTA of k1_filter; >= 1: the filter warps
-// of k1_fused); items first_item, first_item + item_stride, ...  The transaction barriers must have been initialised.
-template <int BAR_ID, int NTHREADS>
+// The CTA: NTHREADS threads; items first_item, first_item + item_stride, ...  The transaction barriers must have been
+// initialised.
+template <int NTHREADS>
 __device__ __forceinline__ void k1_filter_body(const K1SplitParams& q, K1FSmem& sm, const int tid, const int first_item, const int item_stride) {
     const SampleParams& p = q.sp;
     const int lane = tid & 31, warp_id = tid >> 5;
@@ -1304,7 +1302,7 @@ __device__ __forceinline__ void k1_filter_body(const K1SplitParams& q, K1FSmem& 
         }
         __syncwarp();
         if (nframe != frame) {   // moving to the other buffer: the one left behind may be overwritten from the next iteration on
-            group_barrier<BAR_ID, NTHREADS>();
+            __syncthreads();
             cur ^= 1;
         }
     }
@@ -1316,47 +1314,7 @@ __global__ void __maxnreg__(K1F_MAXREG) k1_filter(K1SplitParams q) {
     K1FSmem& sm = *reinterpret_cast<K1FSmem*>(k1f_smem_raw);
     if (threadIdx.x == 0) { mbar_init(&sm.mbar[0]); mbar_init(&sm.mbar[1]); }
     __syncthreads();
-    k1_filter_body<0, K1F_THREADS>(q, sm, threadIdx.x, blockIdx.x, gridDim.x);
-}
-
-// ------------------------------------------------------------------ k1_fused
-// The filter of launch set k and the generator of launch set k+1 in ONE persistent CTA per SM, warp-specialised: 12
-// filter warps (fp64 pipe) and 8 generator warps (integer pipe) share the SM's issue slots, so the generation of the next
-// portion costs (almost) no time of its own.  Separate kernels cannot be made co-resident reliably: two filter CTAs use
-// the whole register file.  Here the register file is split by setmaxnreg: the CTA starts at 96 registers per thread
-// (640 x 96 = 60 K), the generator warp groups drop to 56, the filter warp groups rise to 128.
-#ifndef K1X_FILTER_REGS
-#define K1X_FILTER_REGS 128
-#endif
-#ifndef K1X_GEN_REGS
-#define K1X_GEN_REGS 48
-#endif
-// the CTA's register pool is what it was launched with (640 threads x 96); after the split it must hold
-// 384 x K1X_FILTER_REGS + 256 x K1X_GEN_REGS, or setmaxnreg.inc waits for ever
-static_assert(384 * K1X_FILTER_REGS + 256 * K1X_GEN_REGS <= 640 * 96, "k1_fused: register split exceeds the launch allocation");
-constexpr int K1X_FILTER_THREADS = 384, K1X_GEN_THREADS = K1S_THREADS, K1X_THREADS = K1X_FILTER_THREADS + K1X_GEN_THREADS;
-struct K1XSmem {
-    K1FSmem f;
-    K1GSmem g;
-};
-
-__global__ void __launch_bounds__(K1X_THREADS, 1) k1_fused(K1SplitParams qf, K1SplitParams qg) {
-    extern __shared__ __align__(128) unsigned char k1x_smem_raw[];
-    K1XSmem& sm = *reinterpret_cast<K1XSmem*>(k1x_smem_raw);
-    if (threadIdx.x == 0) { mbar_init(&sm.f.mbar[0]); mbar_init(&sm.f.mbar[1]); }
-    __syncthreads();
-    if (threadIdx.x < K1X_FILTER_THREADS) {
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(K1X_FILTER_REGS));
-        k1_filter_body<2, K1X_FILTER_THREADS>(qf, sm.f, threadIdx.x, blockIdx.x, gridDim.x);
-    } else {
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(K1X_GEN_REGS));
-        const int tid = threadIdx.x - K1X_FILTER_THREADS;
-        const int T = qg.sp.T;
-        for (int slot = blockIdx.x; slot < qg.n_slots; slot += gridDim.x) {
-            k1_slot_body<1, K1X_GEN_THREADS, K1X_GEN_THREADS>(qg, sm.g, tid, slot % T, slot / T);
-            group_barrier<1, K1X_GEN_THREADS>();   // the group's shared memory is reused by the next slot
-        }
-    }
+    k1_filter_body<K1F_THREADS>(q, sm, threadIdx.x, blockIdx.x, gridDim.x);
 }
 
 #ifndef K1V_GROUP

@@ -150,11 +150,9 @@ int dsac_device_view_get(dsac_engine* e, dsac_device_view* view);
 #define DSAC_STAGE_ALL 15u
 int dsac_set_stages(dsac_engine* e, uint32_t mask);
 
-/* Tail split of a batch (scheduling only, results are identical): the sampler runs one CTA per (frame, stream) in
- * waves of as many CTAs as the GPU holds; with the split on, the frames of the whole waves run on an internal
- * high-priority stream and the frames of the last, partial wave on the caller's stream, so that scoring / refinement
- * of the former fill the SMs the partial wave leaves idle.  mode 0: off; 1 (default): dsac_forward_device and the
- * blocking dsac_forward; 2: dsac_forward_submit as well.  Environment override at creation: DSAC_TAIL_SPLIT. */
+/* Which calls may split a batch of at least 768 frames into two lanes (scheduling only, results are identical): two
+ * concurrent half-batches, each a complete pass with its own internal streams, whose kernels fill the GPU in each other's
+ * gaps.  mode 0: never; 1 (default): dsac_forward and dsac_forward_device; 2: dsac_forward_submit as well. */
 int dsac_set_tail_split(dsac_engine* e, int32_t mode);
 
 /* Number of kernels the engine launched since creation (bench.py's gpu_launches). */

@@ -77,12 +77,41 @@ def test_kabsch_matches_oracle(engine_mod, oracle):
     a[0, :, 2] *= 1e-3                    # thin slab: third singular value 1e-6 of the first, still well defined
     b[0] = a[0] @ R0[0].T + t0[0]
     eng = E.Engine(max_frames=1)
-    R, t = eng.kabsch(a, b)
-    for i in range(n):
-        Ro, to = O.kabsch(a[i], b[i])
-        assert np.abs(R[i] - Ro).max() <= (1e-6 if i == 0 else 1e-9)
-        assert np.abs(t[i] - to).max() <= (1e-4 if i == 0 else 1e-7)
-        assert abs(np.linalg.det(R[i]) - 1) < 1e-9
+
+    def check(R, t):
+        for i in range(n):
+            Ro, to = O.kabsch(a[i], b[i])
+            assert np.abs(R[i] - Ro).max() <= (1e-6 if i == 0 else 1e-9)
+            assert np.abs(t[i] - to).max() <= (1e-4 if i == 0 else 1e-7)
+            assert abs(np.linalg.det(R[i]) - 1) < 1e-9
+
+    check(*eng.kabsch(a, b))
+    # the score seam's gradient block is allocated between two kabsch calls of the same size: the second call must still
+    # find its own block intact, and the engine must close cleanly
+    import torch
+
+    class _W:
+        def __init__(self, ptr, shape, typestr):
+            self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
+
+    def bwd_analytic(dm, sg, nf, Hh, out, stream):
+        with torch.cuda.stream(torch.cuda.ExternalStream(stream)):
+            d = torch.as_tensor(_W(dm, (nf, Hh, 1600), "<f4"), device="cuda").double()
+            g = torch.as_tensor(_W(sg, (nf, Hh), "<f8"), device="cuda")
+            o = torch.as_tensor(_W(out, (nf, Hh, 1600), "<f8"), device="cuda")
+            s = torch.sigmoid(0.5 * (10.0 - d))
+            o.copy_(g[:, :, None] * (-0.1 * 0.5) * s * (1 - s))
+        return 0
+
+    coords, pix, gt_cv, gt_jp = E.synth_frames(1)
+    eng.set_score_hook(lambda dm, nf, Hh, sc, stream: 0)
+    eng.set_score_backward_hook(bwd_analytic)
+    eng.forward(coords, pix, gt_jp)
+    bw = eng.backward(coords, pix, gt_jp, full=False)
+    assert np.isfinite(bw.dloss_dobj).all()
+    check(*eng.kabsch(a, b))
+    eng.close()
+    torch.cuda.synchronize()
 
 
 @pytest.mark.parametrize("H", [16, 48])

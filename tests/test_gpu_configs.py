@@ -235,17 +235,17 @@ def test_score_seam_adjoint_hook(engine_mod):
         assert np.abs(got.dloss_dobj[f] - want.dloss_dobj[f]).max() > 0                      # ... and it really took the hook's path
 
 
-def test_two_lanes_are_scheduling_only(engine_mod, monkeypatch):
+def test_two_lanes_are_scheduling_only(engine_mod):
     """A batch of >= 768 frames runs as two concurrent half-batches with their own queues, counters and side streams
-    (engine.cu: forward_split, lane 1).  Frames are independent and sampler streams keyed by the global frame index: the results
-    must be those of the single pass, bit for bit."""
+    (engine.cu: forward_split, lane 1); dsac_set_tail_split(0) keeps it in one pass.  Frames are independent and sampler
+    streams keyed by the global frame index: the results must be those of the single pass, bit for bit."""
     E = engine_mod
     nf = 800
     coords, pix, gt_cv, gt_jp = E.synth_frames(nf)
     out = {}
     for lanes in ("1", "0"):
-        monkeypatch.setenv("DSAC_K1_LANES", lanes)
         eng = E.Engine(max_frames=nf)
+        eng.set_tail_split(int(lanes))
         out[lanes] = eng.forward(coords, pix, gt_jp)
         out[lanes + "b"] = eng.forward(coords, pix, gt_jp)      # a second call: the lanes' own acceptance-rate priors are in use
         eng.close()

@@ -314,8 +314,8 @@ def test_submit_wait_equals_blocking_forward(engine_mod):
 
 @pytest.mark.parametrize("T,H,n", [(8, 32, 40), (1, 16, 300)])
 def test_tail_split_is_scheduling_only(engine_mod, T, H, n):
-    """dsac_set_tail_split moves the frames of the sampler's last, partial wave to another stream: every output
-    must be bit-identical with the split off, on (blocking call, device-resident call) and on for submitted passes."""
+    """dsac_set_tail_split decides which calls may run a large batch as two lanes: every output must be bit-identical
+    with the split off, on (blocking call, device-resident call) and on for submitted passes."""
     import torch
     E = engine_mod
     coords, pix, gt_cv, gt_jp = E.synth_frames(n, n_streams=T)

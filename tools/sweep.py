@@ -44,8 +44,6 @@ def run():
     with open(out, "a") as fh:
         for l in libs:
             env = dict(os.environ, DSAC_B200_LIB=os.path.join(VAR, l))
-            if "__co" in l:   # run-time option encoded in the variant name: preferred shared-memory carve-out of k_sample (percent)
-                env["DSAC_K1_CARVEOUT"] = l.split("__co")[1].split(".")[0]
             try:
                 r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "sweep_one.py")], env=env, capture_output=True, text=True, timeout=300)
                 lines = [x for x in r.stdout.splitlines() if x.startswith("SWEEP ")]
